@@ -2,7 +2,7 @@
 """Benchmark of the hot path: pivots/s of the dense revised simplex loop on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--workload C2|C3|C4] [--pivots P]
+                    [--workload C2|C3|C4] [--pivots P] [--dump-outputs DIR]
 
 A "step" is one window of P pivots of the loop at src/v4_cub_reduction.cu:286-359 on
 a synthetic dense LP (oracle/lpgen_dense: A_s ~ U(0,1), b = (n_s/2)U(1,2),
@@ -186,6 +186,23 @@ def bytes_per_pivot(m, n, itemsize=8):
     return itemsize * (2 * m * m + m * (n - m))
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each array as out_dir/<name>.npy in float64 (int32 indices are exact there), so that two
+    builds can be compared output for output on the same seeded LP.  When the arrays exceed DUMP_BYTES together, each
+    keeps the same share of its rows, chosen by a fixed seed."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES and len(a) > 1:
+            keep = max(1, len(a) * DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(SEED).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled DURING the timed region."""
     Q = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,"
@@ -292,7 +309,11 @@ def run_b200_single(args, wl):
     value = pivots_timed / (total_ms * 1e-3)
     status_after = int(r["status"])
     grid = eng.grid_ctas
-    parity = parity_fields(args.workload, P, eng.trace(P), r["z"])
+    trace = eng.trace(P)
+    parity = parity_fields(args.workload, P, trace, r["z"])
+    if args.dump_outputs:
+        x_b, b_ixs, y = eng.download()      # the state the last timed window left: what b200lp_download hands a caller
+        dump_outputs(args.dump_outputs, {"x_b": x_b, "b_ixs": b_ixs, "y": y, "trace": trace, "z": [r["z"]]})
     eng.close()
 
     # ---- end to end through the C ABI with host buffers ("e2e")
@@ -529,7 +550,14 @@ def main():
     ap.add_argument("--no-km", action="store_true", help="skip the Klee-Minty 20 solve (config 5a) under 'extra'")
     ap.add_argument("--ref-cpu", action="store_true", help="reference arm: force the CPU port")
     ap.add_argument("--ref-pivots", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write x_b, b_ixs, y, the (p, q) trace and z of the last timed window "
+                         "of --workload as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -553,7 +581,7 @@ def main():
             extra["cpu"] = cpu_extras()
         for name in [x for x in args.extras.split(",") if x and x != args.workload]:
             sub = argparse.Namespace(**vars(args))
-            sub.workload, sub.pivots, sub.no_e2e = name, 0, True
+            sub.workload, sub.pivots, sub.no_e2e, sub.dump_outputs = name, 0, True, None
             r = run_b200_single(sub, WORKLOADS[name])
             extra[name] = {k: r[k] for k in ("value", "unit", "ms_per_step", "roofline", "config", "device_loop", "clocks",
                                              "gpu_launches", "trace_sha256", "z_after_window", "trace_matches_golden") if k in r}
