@@ -130,6 +130,38 @@ int b200lp_solve_f32_multi(const float* A, const float* b, const float* c, int64
 		const b200lp_options* opt, const int32_t* devices, int32_t ndev, float* x_b, int32_t* b_ixs,
 		int32_t* trace_pq, int64_t trace_cap, b200lp_result* res);
 
+/*
+ * Many independent LPs of ONE shape in one call (scenario subproblems, parameter sweeps, per-sample LPs).
+ *
+ * Layout: A is `batch` consecutive column-major m x n matrices (leading dimension m), b is batch x m, c is
+ * batch x n.  x_b, b_ixs and y are batch x m; trace_pq is batch x trace_cap x 2 ints, entries past an LP's
+ * pivots are -1.  y and trace_pq may be NULL; a non-NULL trace_pq with trace_cap = 0 receives nothing.
+ * res points to `batch` records: status, iterations, pivots, z and min_reduced_cost are LP k's, aborted is 0;
+ * ms_upload / ms_solve / ms_download / kernel_launches are the whole call's, repeated in every record.
+ * max_iter applies to every LP on its own; check_slack decides per LP whether its last m columns are priced as
+ * unit vectors (identity) or stored like the rest (data), as in the single call.
+ *
+ * Contract: record k and row k of every output are bit-identical to b200lp_solve_f64 / _f32 called on LP k alone
+ * with the same options (y: to b200lp_download after such a run).
+ *
+ * Selection: the LPs run in simplex_tiny_batch (one CTA per LP, persistent grid, all of an LP in shared memory)
+ * when m <= 64 (f64) / 128 (f32), A, B^-1 and the vectors of the LP with the most stored columns fit in 200 KB
+ * of shared memory, pricing_rule = 0, ratio_mode != 2 and max_iter > 0.  Otherwise they run one after another on
+ * one engine (the single call's path without its per-call allocation), so the call accepts every shape and option
+ * b200lp_solve_* accepts.  The single-engine tuning options grid_ctas, tile_shape, mode, profile, price_cols,
+ * price_mode, price_tail, fuse_book2, fuse_ratio, ratio_group_rows, resident and l2_persist_mb affect only that
+ * fallback; eps, max_iter, device, check_slack, pivot_tol, pricing_rule, ratio_mode and harris_delta apply to both.
+ *
+ * Argument errors (B200LP_ERR_ARG, before any device call): batch <= 0, m <= 0, m > n, NULL A / b / c / x_b /
+ * b_ixs / res, trace_cap < 0.  No device: B200LP_ERR_NO_GPU.
+ */
+int b200lp_solve_batch_f64(const double* A, const double* b, const double* c, int64_t batch, int64_t m, int64_t n,
+		const b200lp_options* opt, double* x_b, int32_t* b_ixs, double* y,
+		int32_t* trace_pq, int64_t trace_cap, b200lp_result* res);
+int b200lp_solve_batch_f32(const float* A, const float* b, const float* c, int64_t batch, int64_t m, int64_t n,
+		const b200lp_options* opt, float* x_b, int32_t* b_ixs, float* y,
+		int32_t* trace_pq, int64_t trace_cap, b200lp_result* res);
+
 /* Keep the device buffers of the last b200lp_solve_* call for the next call of the same shape, dtype and options
  * (on != 0), or release them and go back to the reference's behaviour of leaving nothing behind (on == 0, the
  * default).  Creating and freeing 16 GB of device memory costs 40-500 ms per call at m = 32768.  Returns the

@@ -25,6 +25,7 @@ EXPORTS = [
     "b200lp_profile_stamps", "b200lp_profile_names", "b200lp_download_profile", "b200lp_check_basis",
     "b200lp_solve_f64_multi", "b200lp_solve_f32_multi", "b200lp_create_multi", "b200lp_abort",
     "b200lp_refactor", "b200lp_run_guarded", "b200lp_sizeof_options", "b200lp_sizeof_result",
+    "b200lp_solve_batch_f64", "b200lp_solve_batch_f32",
     # include/b200lp_io.h
     "b200lp_read_lp", "b200lp_write_lp_text", "b200lp_write_lp_binary", "b200lp_free_problem",
 ]
@@ -77,6 +78,8 @@ def lib() -> C.CDLL:
         "b200lp_solve_f32": (C.c_int, [vp, vp, vp, i64, i64, PO, vp, vp, vp, i64, PR]),
         "b200lp_solve_f64_multi": (C.c_int, [vp, vp, vp, i64, i64, PO, C.POINTER(i32), i32, vp, vp, vp, i64, PR]),
         "b200lp_solve_f32_multi": (C.c_int, [vp, vp, vp, i64, i64, PO, C.POINTER(i32), i32, vp, vp, vp, i64, PR]),
+        "b200lp_solve_batch_f64": (C.c_int, [vp, vp, vp, i64, i64, i64, PO, vp, vp, vp, vp, i64, vp]),
+        "b200lp_solve_batch_f32": (C.c_int, [vp, vp, vp, i64, i64, i64, PO, vp, vp, vp, vp, i64, vp]),
         "b200lp_create_multi": (C.c_int, [i32, i64, i64, C.POINTER(i32), i32, PO, C.POINTER(vp)]),
         "b200lp_abort": (C.c_int, [vp]),
         "b200lp_refactor": (C.c_int, [vp, dbl, C.POINTER(i64)]),

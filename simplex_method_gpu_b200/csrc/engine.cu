@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -73,10 +74,21 @@ struct b200lp_engine {
 namespace {
 
 template <typename T> class MultiEngine;
+template <typename T> class BatchCall;
+
+// tiny LPs: ld is one warp-wide vector row (m <= 64 doubles / 128 floats) and A (ns stored columns), B^-1 and the
+// vectors fit in one CTA's shared memory.  Asked by the single engine (simplex_tiny) and by the batched call
+// (simplex_tiny_batch, ns = the largest of the batch).
+template <typename T>
+bool tiny_fits(long long m, long long n, long long ns) {
+	if (m > TinyLayout<T>::LD) return false;
+	return TinyLayout<T>(m, n, ns).bytes(m) <= (size_t)200 * 1024;
+}
 
 template <typename T>
 class Engine final : public b200lp_engine {
 	friend class MultiEngine<T>;
+	friend class BatchCall<T>;
 public:
 	Engine(int64_t m, int64_t n, const b200lp_options& o, int rank_, int nranks_) : opt(o) {
 		std::memset(&d, 0, sizeof(d));
@@ -922,8 +934,7 @@ private:
 	// Only with the automatic grid: an explicit grid_ctas asks for the general kernel.
 	bool tiny_ok() const {
 		if (nranks != 1 || opt.grid_ctas > 0 || opt.mode != 0 || d.prof_cap > 0 || opt.pricing_rule != 0 || opt.ratio_mode == 2) return false;
-		if (d.ld != 32 * VecT<T>::N) return false;
-		return TinyLayout<T>(d.m, d.n, d.ns).bytes(d.m) <= (size_t)200 * 1024;
+		return tiny_fits<T>(d.m, d.n, d.ns);
 	}
 
 	// mid-size LPs whose A and B^-1 fit in the shared memory of the whole grid (one CTA per SM): the resident kernel.
@@ -1418,6 +1429,205 @@ int solve_once(const T* A, const T* b, const T* c, int64_t m, int64_t n, const b
 	return rc;
 }
 
+// Many LPs of one shape in one call (b200lp_solve_batch_*).  Tiny shapes with the Dantzig rule and a one-pass ratio
+// test run in simplex_tiny_batch (one CTA per LP, a persistent grid fed by a ticket counter); everything else runs
+// the LPs one after another on one engine (upload, run, download per LP).  Either way record k and row k of every
+// output are bit-identical to b200lp_solve_* on LP k alone.
+template <typename T>
+class BatchCall {
+public:
+	BatchCall(const T* A, const T* b, const T* c, int64_t batch, int64_t m, int64_t n, const b200lp_options& o,
+			T* x_b, int32_t* b_ixs, T* y, int32_t* trace_pq, int64_t trace_cap, b200lp_result* res)
+		: A(A), b(b), c(c), batch(batch), m(m), n(n), o(o), x_b(x_b), b_ixs(b_ixs), y(y), trace_pq(trace_pq),
+		  trace_cap(trace_pq ? trace_cap : 0), res(res) {}
+
+	~BatchCall() {
+		for (void* p : owned) cudaFree(p);
+		if (stream) cudaStreamDestroy(stream);
+		for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
+	}
+
+	int run() {
+		// structural columns per LP: the rule of Engine::upload (check_slack), slack blocks checked on host threads
+		std::vector<int> ns((size_t)batch);
+		{
+			const unsigned nt = (unsigned)std::max<int64_t>(1, std::min<int64_t>(std::max(1u, std::thread::hardware_concurrency()), batch));
+			auto work = [&](int64_t k0, int64_t k1) {
+				for (int64_t k = k0; k < k1; ++k)
+					ns[k] = (int)(!o.check_slack || Engine<T>::host_is_identity(A + (size_t)k * m * n + (size_t)(n - m) * m, m) ? n - m : n);
+			};
+			std::vector<std::thread> th;
+			for (unsigned t = 0; t < nt; ++t) th.emplace_back(work, batch * t / nt, batch * (t + 1) / nt);
+			for (auto& t : th) t.join();
+		}
+		const int ns_max = *std::max_element(ns.begin(), ns.end());
+		if (o.max_iter > 0 && o.pricing_rule == 0 && o.ratio_mode != 2 && tiny_fits<T>(m, n, ns_max)) return run_kernel(ns, ns_max);
+		return run_engine();
+	}
+
+private:
+	template <typename U>
+	cudaError_t alloc(U** p, size_t count) {
+		void* v = nullptr;
+		cudaError_t e = cudaMalloc(&v, std::max<size_t>(count, 1) * sizeof(U));
+		if (e == cudaSuccess) owned.push_back(v);
+		*p = static_cast<U*>(v);
+		return e;
+	}
+
+	int run_kernel(const std::vector<int>& ns, int ns_max) {
+		CU(cudaSetDevice(o.device));
+		cudaDeviceProp prop;
+		CU(cudaGetDeviceProperties(&prop, o.device));
+		if (prop.major < 10)
+			return fail(B200LP_ERR_NO_GPU, std::string("device is sm_") + std::to_string(prop.major * 10 + prop.minor) +
+				", the engine is built for sm_100a only");
+		CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+		for (auto& e : ev) CU(cudaEventCreate(&e));
+		const size_t bm = (size_t)batch * m, bn = (size_t)batch * n;
+		TinyBatch<T> bt;
+		std::memset(&bt, 0, sizeof(bt));
+		T *dA, *db, *dc, *dx, *dy = nullptr;
+		int *dns, *dbix;
+		int2* dtr = nullptr;
+		TinyBatchRec* drec;
+		unsigned long long* dticket;
+		CU(alloc(&dA, bm * n));
+		CU(alloc(&db, bm));
+		CU(alloc(&dc, bn));
+		CU(alloc(&dns, (size_t)batch));
+		CU(alloc(&dx, bm));
+		CU(alloc(&dbix, bm));
+		if (y) CU(alloc(&dy, bm));
+		if (trace_cap > 0) CU(alloc(&dtr, (size_t)batch * trace_cap));
+		CU(alloc(&drec, (size_t)batch));
+		CU(alloc(&dticket, 1));
+		CU(cudaEventRecord(ev[0], stream));
+		CU(cudaMemcpyAsync(dA, A, bm * n * sizeof(T), cudaMemcpyHostToDevice, stream));
+		CU(cudaMemcpyAsync(db, b, bm * sizeof(T), cudaMemcpyHostToDevice, stream));
+		CU(cudaMemcpyAsync(dc, c, bn * sizeof(T), cudaMemcpyHostToDevice, stream));
+		CU(cudaMemcpyAsync(dns, ns.data(), (size_t)batch * sizeof(int), cudaMemcpyHostToDevice, stream));
+		CU(cudaMemsetAsync(dticket, 0, sizeof(unsigned long long), stream));
+		if (dtr) CU(cudaMemsetAsync(dtr, 0xff, (size_t)batch * trace_cap * sizeof(int2), stream));   // -1: no pivot
+		CU(cudaEventRecord(ev[1], stream));
+
+		bt.batch = batch; bt.m = m; bt.n = n;
+		bt.A = dA; bt.b = db; bt.c = dc; bt.ns = dns;
+		bt.it_end = o.max_iter;
+		bt.eps = sizeof(T) == 4 ? (double)(float)o.eps : o.eps;                  // as Engine does
+		bt.pivot_tol = sizeof(T) == 4 ? (double)(float)o.pivot_tol : o.pivot_tol;
+		bt.ratio_mode = o.ratio_mode;
+		bt.x_b = dx; bt.y = dy; bt.b_ixs = dbix; bt.trace = dtr; bt.trace_cap = trace_cap; bt.rec = drec; bt.ticket = dticket;
+		const size_t smem = TinyLayout<T>(m, n, ns_max).bytes(m);
+		CU(cudaFuncSetAttribute(simplex_tiny_batch<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+		int occ = 0;
+		CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_tiny_batch<T>, NT, smem));
+		if (occ < 1) return fail(B200LP_ERR_CUDA, "simplex_tiny_batch does not fit on an SM");
+		const int grid = (int)std::min<int64_t>(batch, (int64_t)occ * prop.multiProcessorCount);
+		simplex_tiny_batch<T><<<grid, NT, smem, stream>>>(bt);
+		CU(cudaGetLastError());
+		CU(cudaEventRecord(ev[2], stream));
+
+		std::vector<TinyBatchRec> rec((size_t)batch);
+		CU(cudaMemcpyAsync(rec.data(), drec, (size_t)batch * sizeof(TinyBatchRec), cudaMemcpyDeviceToHost, stream));
+		CU(cudaMemcpyAsync(x_b, dx, bm * sizeof(T), cudaMemcpyDeviceToHost, stream));
+		CU(cudaMemcpyAsync(b_ixs, dbix, bm * sizeof(int), cudaMemcpyDeviceToHost, stream));
+		if (y) CU(cudaMemcpyAsync(y, dy, bm * sizeof(T), cudaMemcpyDeviceToHost, stream));
+		if (dtr) CU(cudaMemcpyAsync(trace_pq, dtr, (size_t)batch * trace_cap * sizeof(int2), cudaMemcpyDeviceToHost, stream));
+		CU(cudaEventRecord(ev[3], stream));
+		CU(cudaStreamSynchronize(stream));
+		float up = 0, solve = 0, down = 0;
+		CU(cudaEventElapsedTime(&up, ev[0], ev[1]));
+		CU(cudaEventElapsedTime(&solve, ev[1], ev[2]));
+		CU(cudaEventElapsedTime(&down, ev[2], ev[3]));
+		for (int64_t k = 0; k < batch; ++k) {
+			b200lp_result& r = res[k];
+			std::memset(&r, 0, sizeof(r));
+			r.status = rec[k].status;
+			r.iterations = rec[k].iterations;
+			r.pivots = rec[k].pivots;
+			r.z = rec[k].z;
+			r.min_reduced_cost = rec[k].min_e;
+			r.ms_upload = up;
+			r.ms_solve = solve;
+			r.ms_download = down;
+			r.kernel_launches = 1;
+		}
+		return B200LP_OK;
+	}
+
+	// any other shape or option: the LPs one after another on one engine, i.e. exactly the single call's path
+	int run_engine() {
+		b200lp_engine* e = nullptr;
+		if (int rc = create_engine<T>(m, n, &o, &e)) return rc;
+		std::unique_ptr<b200lp_engine> own(e);
+		double up = 0, solve = 0, down = 0;
+		using Clk = std::chrono::steady_clock;
+		for (int64_t k = 0; k < batch; ++k) {
+			b200lp_result& r = res[k];
+			if (int rc = e->upload(A + (size_t)k * m * n, b + (size_t)k * m, c + (size_t)k * n)) return rc;
+			if (int rc = e->run_async(o.max_iter)) return rc;
+			if (int rc = e->wait(&r)) return rc;
+			const auto t = Clk::now();
+			if (int rc = e->download(x_b + (size_t)k * m, b_ixs + (size_t)k * m, y ? y + (size_t)k * m : nullptr)) return rc;
+			if (trace_cap > 0) {
+				int32_t* tr = trace_pq + (size_t)k * trace_cap * 2;
+				int64_t got = 0;
+				if (int rc = e->download_trace(tr, trace_cap, &got)) return rc;
+				std::fill(tr + 2 * got, tr + 2 * trace_cap, -1);
+			}
+			down += std::chrono::duration<double, std::milli>(Clk::now() - t).count();
+			up += r.ms_upload;
+			solve += r.ms_solve;
+		}
+		const int64_t launches = res[batch - 1].kernel_launches;    // the engine's count covers the whole call
+		for (int64_t k = 0; k < batch; ++k) {
+			res[k].aborted = 0;
+			res[k].ms_upload = up;
+			res[k].ms_solve = solve;
+			res[k].ms_download = down;
+			res[k].kernel_launches = launches;
+		}
+		return B200LP_OK;
+	}
+
+	const T *A, *b, *c;
+	int64_t batch, m, n;
+	b200lp_options o;
+	T* x_b;
+	int32_t* b_ixs;
+	T* y;
+	int32_t* trace_pq;
+	int64_t trace_cap;
+	b200lp_result* res;
+	std::vector<void*> owned;
+	cudaStream_t stream = nullptr;
+	cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+};
+
+template <typename T>
+int solve_batch(const T* A, const T* b, const T* c, int64_t batch, int64_t m, int64_t n, const b200lp_options* opt,
+		T* x_b, int32_t* b_ixs, T* y, int32_t* trace_pq, int64_t trace_cap, b200lp_result* res) {
+	if (batch <= 0) return fail(B200LP_ERR_ARG, "batch must be positive");
+	if (m <= 0 || n <= 0 || m > n) return fail(B200LP_ERR_ARG, "need 0 < m <= n (v4:402)");
+	if (n >= ((int64_t)1 << 31)) return fail(B200LP_ERR_ARG, "n must fit a 32-bit basis index");
+	if (!A || !b || !c) return fail(B200LP_ERR_ARG, "A, b, c must not be NULL");
+	if (!x_b || !b_ixs || !res) return fail(B200LP_ERR_ARG, "x_b, b_ixs, res must not be NULL");
+	if (trace_cap < 0) return fail(B200LP_ERR_ARG, "trace_cap must not be negative");
+	b200lp_options o;
+	if (opt) o = *opt; else b200lp_default_options(&o);
+	if (o.pricing_rule != 0 && o.pricing_rule != 1) return fail(B200LP_ERR_ARG, "pricing_rule must be 0 (Dantzig) or 1 (steepest edge)");
+	if (o.ratio_mode < 0 || o.ratio_mode > 2) return fail(B200LP_ERR_ARG, "ratio_mode must be 0, 1 or 2");
+	int ndev = 0;
+	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+		cudaGetLastError();
+		return fail(B200LP_ERR_NO_GPU, "no CUDA device: the engine has no CPU fallback");
+	}
+	if (o.device < 0 || o.device >= ndev) return fail(B200LP_ERR_ARG, "device ordinal out of range");
+	BatchCall<T> call(A, b, c, batch, m, n, o, x_b, b_ixs, y, trace_pq, trace_cap, res);
+	return call.run();
+}
+
 } // namespace
 
 // host-side twin of k_generate_dense (same counter-based numbers), threaded over columns
@@ -1476,6 +1686,18 @@ int b200lp_solve_f64(const double* A, const double* b, const double* c, int64_t 
 int b200lp_solve_f32(const float* A, const float* b, const float* c, int64_t m, int64_t n,
 		const b200lp_options* opt, float* x_b, int32_t* b_ixs, int32_t* trace_pq, int64_t trace_cap, b200lp_result* res) {
 	return solve_once<float>(A, b, c, m, n, opt, x_b, b_ixs, trace_pq, trace_cap, res);
+}
+
+int b200lp_solve_batch_f64(const double* A, const double* b, const double* c, int64_t batch, int64_t m, int64_t n,
+		const b200lp_options* opt, double* x_b, int32_t* b_ixs, double* y, int32_t* trace_pq, int64_t trace_cap,
+		b200lp_result* res) {
+	return solve_batch<double>(A, b, c, batch, m, n, opt, x_b, b_ixs, y, trace_pq, trace_cap, res);
+}
+
+int b200lp_solve_batch_f32(const float* A, const float* b, const float* c, int64_t batch, int64_t m, int64_t n,
+		const b200lp_options* opt, float* x_b, int32_t* b_ixs, float* y, int32_t* trace_pq, int64_t trace_cap,
+		b200lp_result* res) {
+	return solve_batch<float>(A, b, c, batch, m, n, opt, x_b, b_ixs, y, trace_pq, trace_cap, res);
 }
 
 int b200lp_solve_f64_multi(const double* A, const double* b, const double* c, int64_t m, int64_t n,

@@ -1507,40 +1507,34 @@ struct TinyLayout {
 	__host__ __device__ size_t bytes(long long m) const { return (size_t)end * sizeof(T) + (size_t)m * sizeof(int) + 16; }
 };
 
+// Shared-memory pointers of one tiny LP (TinyLayout) and its sizes.
 template <typename T>
-__global__ void __launch_bounds__(NT, 1) simplex_tiny(Dev<T> d) {
+struct TinyLP {
+	T *A, *B, *y, *x_b, *c_b, *alpha, *E_q, *row_q, *b, *part, *c;
+	int* b_ixs;
+	int m, n, ns;
+	__device__ __forceinline__ TinyLP(T* S, const TinyLayout<T>& L, int m_, int n_, int ns_)
+		: A(S + L.A), B(S + L.B), y(S + L.y), x_b(S + L.x_b), c_b(S + L.c_b), alpha(S + L.alpha), E_q(S + L.E_q),
+		  row_q(S + L.row_q), b(S + L.b), part(S + L.part), c(S + L.c), b_ixs(reinterpret_cast<int*>(S + L.end)),
+		  m(m_), n(n_), ns(ns_) {}
+};
+
+// The pivot loop of the tiny kernels (simplex_tiny, simplex_tiny_batch): iterations [it, it_end) on the LP in
+// shared memory, the scalar state in registers of every thread.  Leaves after the last iteration or at
+// optimum / unbounded (status, done set, the final iteration counted like the general kernel does).
+template <typename T>
+__device__ __forceinline__ void tiny_pivots(const TinyLP<T>& s, Smem& sh, double eps, double pivot_tol, int ratio_mode,
+		int2* trace, long long trace_cap, long long& it, const long long it_end, long long& pivots, int& pending,
+		int& status, int& done, long long& p, long long& q, double& min_e) {
 	using V = typename VecT<T>::V;
 	using M = Mem<T>;
 	constexpr int VN = VecT<T>::N;
 	constexpr int LD = 32 * VN;
-	__shared__ Smem sh;
-	extern __shared__ __align__(128) unsigned char dynraw[];
-	T* S = reinterpret_cast<T*>(dynraw);
-	const TinyLayout<T> L(d.m, d.n, d.ns);
-	T *sA = S + L.A, *sB = S + L.B, *sy = S + L.y, *sx = S + L.x_b, *scb = S + L.c_b, *sal = S + L.alpha,
-	  *sE = S + L.E_q, *srq = S + L.row_q, *sb = S + L.b, *spart = S + L.part, *sc = S + L.c;
-	int* sbix = reinterpret_cast<int*>(S + L.end);
+	T *sA = s.A, *sB = s.B, *sy = s.y, *sx = s.x_b, *scb = s.c_b, *sal = s.alpha, *sE = s.E_q, *srq = s.row_q,
+	  *sb = s.b, *spart = s.part, *sc = s.c;
+	int* sbix = s.b_ixs;
 	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-	const int m = (int)d.m, n = (int)d.n, ns = (int)d.ns;
-	Ctl* ctl = d.ctl;
-
-	// ---- state in
-	for (long long e = tid; e < (long long)LD * ns; e += NT) sA[e] = d.A[e];
-	for (long long e = tid; e < (long long)LD * m; e += NT) sB[e] = d.B[e];
-	for (int i = tid; i < LD; i += NT) {
-		sy[i] = d.y[i]; sx[i] = d.x_b[i]; scb[i] = d.c_b[i]; sal[i] = d.alpha[i];
-		sE[i] = d.E_q[i]; srq[i] = d.row_q[i]; sb[i] = d.b[i];
-	}
-	for (int j = tid; j < n; j += NT) sc[j] = d.c[j];
-	for (int i = tid; i < m; i += NT) sbix[i] = d.b_ixs[i];
-	long long it = ctl->iter, pivots = ctl->pivots;
-	const long long it_end = ctl->it_end;
-	int pending = ctl->pending;
-	int status = 0, done = 0;
-	long long p = ctl->p, q = ctl->q;
-	double min_e = ctl->min_e;
-	__syncthreads();
-
+	const int m = s.m, n = s.n, ns = s.ns;
 	while (it < it_end) {
 		// ---- pricing (v4:288-302): warp w takes columns w, w+8, ...; the column's 32 vectors are this warp's lanes
 		double best_v = CUDART_INF;
@@ -1563,7 +1557,7 @@ __global__ void __launch_bounds__(NT, 1) simplex_tiny(Dev<T> d) {
 		block_argmin(best_v, best_i, sh);
 		min_e = best_v;
 		p = best_i;
-		if (min_e >= -d.eps) { status = 1; done = 1; ++it; break; }
+		if (min_e >= -eps) { status = 1; done = 1; ++it; break; }
 
 		// ---- pending rank-1 update fused with the FTRAN of column p (v4:333 + v4:307-308)
 		{
@@ -1613,9 +1607,9 @@ __global__ void __launch_bounds__(NT, 1) simplex_tiny(Dev<T> d) {
 		long long elig = 0;
 		for (int i = tid; i < m; i += NT) {
 			const T a = sal[i];
-			if (a > (T)d.pivot_tol) {
+			if (a > (T)pivot_tol) {
 				++elig;
-				const double th = (double)(ratio_num(sx[i], d.ratio_mode) / a);
+				const double th = (double)(ratio_num(sx[i], ratio_mode) / a);
 				if (cand_better(th, i, best_v, best_i)) { best_v = th; best_i = i; }
 			}
 		}
@@ -1661,12 +1655,65 @@ __global__ void __launch_bounds__(NT, 1) simplex_tiny(Dev<T> d) {
 			sy[i] = fma_t(syv, rq, sy[i]);
 			if (i == q) { scb[i] = c_p; sbix[i] = (int)p; }
 		}
-		if (tid == 0 && pivots < d.trace_cap) d.trace[pivots] = make_int2((int)p, (int)q);
+		if (tid == 0 && pivots < trace_cap) trace[pivots] = make_int2((int)p, (int)q);
 		pending = 1;
 		++pivots;
 		++it;
 		__syncthreads();
 	}
+}
+
+// z = c_b . x_b in slice order (v4:365); the sum is valid in thread 0
+template <typename T>
+__device__ __forceinline__ T tiny_objective(const T* scb, const T* sx, int m, Smem& sh) {
+	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	T t = tid < m ? fma_t(scb[tid], sx[tid], T(0)) : T(0);
+	t = warp_butterfly_sum(t);
+	__syncthreads();
+	if (lane == 0) sh.dsum[0][warp] = (double)t;
+	__syncthreads();
+	T a = T(0);
+	if (tid == 0) {
+#pragma unroll
+		for (int w = 0; w < NWARP; ++w) a = a + (T)sh.dsum[0][w];
+	}
+	return T(0) + a;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(NT, 1) simplex_tiny(Dev<T> d) {
+	constexpr int LD = TinyLayout<T>::LD;
+	__shared__ Smem sh;
+	extern __shared__ __align__(128) unsigned char dynraw[];
+	T* S = reinterpret_cast<T*>(dynraw);
+	const TinyLayout<T> L(d.m, d.n, d.ns);
+	const TinyLP<T> s(S, L, (int)d.m, (int)d.n, (int)d.ns);
+	T *sA = s.A, *sB = s.B, *sy = s.y, *sx = s.x_b, *scb = s.c_b, *sal = s.alpha, *sE = s.E_q, *srq = s.row_q, *sb = s.b,
+	  *sc = s.c;
+	int* sbix = s.b_ixs;
+	const int tid = threadIdx.x;
+	const int m = (int)d.m, n = (int)d.n, ns = (int)d.ns;
+	Ctl* ctl = d.ctl;
+
+	// ---- state in
+	for (long long e = tid; e < (long long)LD * ns; e += NT) sA[e] = d.A[e];
+	for (long long e = tid; e < (long long)LD * m; e += NT) sB[e] = d.B[e];
+	for (int i = tid; i < LD; i += NT) {
+		sy[i] = d.y[i]; sx[i] = d.x_b[i]; scb[i] = d.c_b[i]; sal[i] = d.alpha[i];
+		sE[i] = d.E_q[i]; srq[i] = d.row_q[i]; sb[i] = d.b[i];
+	}
+	for (int j = tid; j < n; j += NT) sc[j] = d.c[j];
+	for (int i = tid; i < m; i += NT) sbix[i] = d.b_ixs[i];
+	long long it = ctl->iter, pivots = ctl->pivots;
+	const long long it_end = ctl->it_end;
+	int pending = ctl->pending;
+	int status = 0, done = 0;
+	long long p = ctl->p, q = ctl->q;
+	double min_e = ctl->min_e;
+	__syncthreads();
+
+	tiny_pivots(s, sh, d.eps, d.pivot_tol, d.ratio_mode, d.trace, d.trace_cap, it, it_end, pivots, pending, status, done,
+		p, q, min_e);
 
 	// ---- state out
 	__syncthreads();
@@ -1675,20 +1722,108 @@ __global__ void __launch_bounds__(NT, 1) simplex_tiny(Dev<T> d) {
 		d.y[k] = sy[k]; d.x_b[k] = sx[k]; d.c_b[k] = scb[k]; d.alpha[k] = sal[k]; d.E_q[k] = sE[k]; d.row_q[k] = srq[k];
 	}
 	for (int k = tid; k < m; k += NT) d.b_ixs[k] = sbix[k];
-	// z = c_b . x_b in slice order (v4:365)
-	T t = tid < m ? fma_t(scb[tid], sx[tid], T(0)) : T(0);
-	t = warp_butterfly_sum(t);
-	__syncthreads();
-	if (lane == 0) sh.dsum[0][warp] = (double)t;
-	__syncthreads();
+	const T z = tiny_objective(scb, sx, m, sh);
 	if (tid == 0) {
-		T a = T(0);
-#pragma unroll
-		for (int w = 0; w < NWARP; ++w) a = a + (T)sh.dsum[0][w];
-		const T z = T(0) + a;
 		ctl->iter = it; ctl->pivots = pivots; ctl->pending = pending;
 		ctl->status = status; ctl->done = done;
 		ctl->p = p; ctl->q = q; ctl->min_e = min_e; ctl->z = (double)z; ctl->c_b_q = sh.bc_v;
+	}
+}
+
+// ---------------------------------------------------------------- many tiny LPs of one shape: one CTA per LP
+//
+// b200lp_solve_batch_*: the LPs of a batch are independent, so every CTA of a persistent grid solves whole LPs
+// with the loop of simplex_tiny (tiny_pivots, NT threads, the same summation orders: the same bits as a single
+// call).  CTAs take LP indices from a ticket counter because pivot counts differ by orders of magnitude between
+// LPs; the order of hand-out changes no bit.  Each LP starts from the slack basis built in shared memory exactly
+// as upload / reset leave it for simplex_tiny (k_reset); nothing per LP lives in HBM besides inputs and outputs.
+constexpr int TINY_BATCH_MIN_CTAS = 2;   // 104 registers x 256 threads (f64): two CTAs per SM by registers
+
+// one LP's outcome (the per-LP fields of b200lp_result)
+struct TinyBatchRec {
+	long long iterations, pivots;
+	double z, min_e;
+	int status, pad;
+};
+
+template <typename T>
+struct TinyBatch {
+	long long batch, m, n;
+	const T* A;               // batch x (m x n column-major, leading dimension m)
+	const T* b;               // batch x m
+	const T* c;               // batch x n
+	const int* ns;            // structural (stored, priced as dense) columns of every LP: n - m or n
+	long long it_end;         // max_iter, per LP
+	double eps, pivot_tol;
+	int ratio_mode;
+	T* x_b;                   // batch x m
+	T* y;                     // batch x m, or null
+	int* b_ixs;               // batch x m
+	int2* trace;              // batch x trace_cap (p, q), or null
+	long long trace_cap;
+	TinyBatchRec* rec;        // batch
+	unsigned long long* ticket; // next LP to hand out (zeroed by the host before the launch)
+};
+
+template <typename T>
+__global__ void __launch_bounds__(NT, TINY_BATCH_MIN_CTAS) simplex_tiny_batch(TinyBatch<T> bt) {
+	constexpr int LD = TinyLayout<T>::LD;
+	__shared__ Smem sh;
+	__shared__ long long s_k;
+	extern __shared__ __align__(128) unsigned char dynraw[];
+	T* S = reinterpret_cast<T*>(dynraw);
+	const int tid = threadIdx.x;
+	const int m = (int)bt.m, n = (int)bt.n;
+	for (;;) {
+		if (tid == 0) s_k = (long long)atomicAdd(bt.ticket, 1ULL);
+		__syncthreads();
+		const long long k = s_k;
+		if (k >= bt.batch) break;
+		const int ns = bt.ns[k];
+		const TinyLayout<T> L(m, n, ns);
+		const TinyLP<T> s(S, L, m, n, ns);
+		const T* Ak = bt.A + (size_t)k * (size_t)m * (size_t)n;
+		const T* bk = bt.b + (size_t)k * m;
+		const T* ck = bt.c + (size_t)k * n;
+
+		// ---- state in: the slack basis of k_reset, padding rows +0
+		for (long long e = tid; e < (long long)LD * ns; e += NT) {
+			const int i = (int)(e % LD);
+			s.A[e] = i < m ? Ak[(e / LD) * m + i] : T(0);
+		}
+		for (long long e = tid; e < (long long)LD * m; e += NT) s.B[e] = e % LD == e / LD ? T(1) : T(0);
+		for (int i = tid; i < LD; i += NT) {
+			const bool in = i < m;
+			const T cb = in ? ck[n - m + i] : T(0);
+			const T bi = in ? bk[i] : T(0);
+			s.y[i] = cb; s.c_b[i] = cb; s.x_b[i] = bi; s.b[i] = bi;
+			s.alpha[i] = T(0); s.E_q[i] = T(0); s.row_q[i] = T(0);
+		}
+		for (int j = tid; j < n; j += NT) s.c[j] = ck[j];
+		for (int i = tid; i < m; i += NT) s.b_ixs[i] = n - m + i;
+		long long it = 0, pivots = 0, p = 0, q = 0;
+		int pending = 0, status = 0, done = 0;
+		double min_e = 0;
+		__syncthreads();
+
+		int2* tr = bt.trace ? bt.trace + (size_t)k * bt.trace_cap : nullptr;
+		tiny_pivots(s, sh, bt.eps, bt.pivot_tol, bt.ratio_mode, tr, tr ? bt.trace_cap : 0, it, bt.it_end, pivots, pending,
+			status, done, p, q, min_e);
+
+		// ---- state out
+		__syncthreads();
+		for (int i = tid; i < m; i += NT) {
+			bt.x_b[(size_t)k * m + i] = s.x_b[i];
+			bt.b_ixs[(size_t)k * m + i] = s.b_ixs[i];
+			if (bt.y) bt.y[(size_t)k * m + i] = s.y[i];
+		}
+		const T z = tiny_objective(s.c_b, s.x_b, m, sh);
+		if (tid == 0) {
+			TinyBatchRec r;
+			r.iterations = it; r.pivots = pivots; r.z = (double)z; r.min_e = min_e; r.status = status; r.pad = 0;
+			bt.rec[k] = r;
+		}
+		__syncthreads();                               // shared memory (ticket, LP) is reused by the next LP
 	}
 }
 

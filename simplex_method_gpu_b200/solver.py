@@ -108,6 +108,78 @@ def solve(A, b, c, eps: float = EPS, max_iter: int = MAX_ITER, dtype=None, devic
                     res.ms_upload, res.ms_solve, res.ms_download, res.kernel_launches, res.min_reduced_cost)
 
 
+@dataclass
+class BatchSolution:
+    """Outcome of solve_batch: arrays indexed by LP, the call's timings once."""
+    z: np.ndarray                 # (batch,)
+    status: np.ndarray            # (batch,) int32, SolveStatus values
+    iterations: np.ndarray        # (batch,) int64
+    pivots: np.ndarray            # (batch,) int64
+    min_reduced_cost: np.ndarray  # (batch,)
+    x_b: np.ndarray               # (batch, m) basis-ordered values
+    b_ixs: np.ndarray             # (batch, m) basis-ordered column indices
+    y: np.ndarray | None          # (batch, m) duals, None unless want_y
+    trace: np.ndarray             # (batch, trace_cap, 2) int32 (p, q), -1 past an LP's pivots
+    ms_upload: float = 0.0
+    ms_solve: float = 0.0
+    ms_download: float = 0.0
+    kernel_launches: int = 0
+
+    def __len__(self) -> int:
+        return len(self.z)
+
+    def solution(self, k: int) -> Solution:
+        """LP k as the Solution of a single solve() (format_result works on it)."""
+        k = int(k)
+        piv = int(self.pivots[k])
+        return Solution(float(self.z[k]), SolveStatus(int(self.status[k])), self.x_b[k].copy(), self.b_ixs[k].copy(),
+                        int(self.iterations[k]), piv, self.trace[k, :min(piv, self.trace.shape[1])].copy(),
+                        self.ms_upload, self.ms_solve, self.ms_download, self.kernel_launches,
+                        float(self.min_reduced_cost[k]))
+
+
+def solve_batch(A, b, c, eps: float = EPS, max_iter: int = MAX_ITER, dtype=None, device: int = 0, trace_cap: int = 0,
+                want_y: bool = True, **opts) -> BatchSolution:
+    """Many LPs of one shape in one call (b200lp_solve_batch_*): A is (batch, m, n), b (batch, m), c (batch, n).
+    LP k's results are bit-identical to ``solve(A[k], b[k], c[k], ...)`` with the same options."""
+    A = np.asarray(A)
+    dt = np.dtype(dtype if dtype is not None else A.dtype)
+    _dtype_code(dt)
+    if A.ndim != 3:
+        raise ValueError("A must be a stack of matrices (batch, m, n)")
+    batch, m, n = A.shape
+    At = np.ascontiguousarray(A.transpose(0, 2, 1), dtype=dt)     # every LP column-major (v4:59-60)
+    b = np.ascontiguousarray(b, dtype=dt)
+    c = np.ascontiguousarray(c, dtype=dt)
+    if b.shape != (batch, m) or c.shape != (batch, n):
+        raise ValueError(f"shape mismatch: A is {batch}x{m}x{n}, b is {'x'.join(map(str, b.shape))}, "
+                         f"c is {'x'.join(map(str, c.shape))}")
+    if m > n:
+        raise ValueError("Either failed to read m and n, or m > n.")   # v4:403
+    if batch == 0:
+        raise ValueError("the batch is empty")
+    cap = int(trace_cap)
+    if cap < 0:
+        raise ValueError("trace_cap must not be negative")
+    L = capi.lib()
+    o = capi.default_options(eps=eps, max_iter=int(max_iter), device=device, **opts)
+    x_b = np.zeros((batch, m), dt)
+    b_ixs = np.zeros((batch, m), np.int32)
+    y = np.zeros((batch, m), dt) if want_y else None
+    trace = np.full((batch, cap, 2), -1, np.int32)
+    res = (capi.Result * batch)()
+    fn = L.b200lp_solve_batch_f64 if dt == np.float64 else L.b200lp_solve_batch_f32
+    capi.check(fn(_vp(At), _vp(b), _vp(c), batch, m, n, C.byref(o), _vp(x_b), _vp(b_ixs), _vp(y),
+                  _vp(trace) if cap > 0 else None, cap, res))
+    r0 = res[0]
+    return BatchSolution(z=np.array([r.z for r in res]), status=np.array([r.status for r in res], np.int32),
+                         iterations=np.array([r.iterations for r in res], np.int64),
+                         pivots=np.array([r.pivots for r in res], np.int64),
+                         min_reduced_cost=np.array([r.min_reduced_cost for r in res]),
+                         x_b=x_b, b_ixs=b_ixs, y=y, trace=trace, ms_upload=r0.ms_upload, ms_solve=r0.ms_solve,
+                         ms_download=r0.ms_download, kernel_launches=r0.kernel_launches)
+
+
 def set_memory_cache(on: bool) -> bool:
     """Keep the device buffers of the last solve() for the next call of the same shape (b200lp_set_memory_cache)."""
     return bool(capi.lib().b200lp_set_memory_cache(1 if on else 0))
