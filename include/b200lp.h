@@ -37,6 +37,11 @@ extern "C" {
 #define B200LP_STATUS_OPTIMUM        1
 #define B200LP_STATUS_UNBOUNDED      2
 #define B200LP_STATUS_THETA_OVERFLOW 3 /* unreachable, kept for enum parity (v1 only) */
+/* dual simplex only (options.algorithm = 1): */
+#define B200LP_STATUS_INFEASIBLE     4 /* no entering column for the leaving row r: row r of B^-1 proves Ax <= b,
+                                          x >= 0 infeasible (rho.b = x_b[r] < 0, rho.a_j >= 0 for every nonbasic j) */
+#define B200LP_STATUS_NOT_DUAL_FEASIBLE 5 /* some reduced cost e_j < -eps: the dual method cannot start (or continue)
+                                          from this basis; the primal method (algorithm = 0) applies */
 
 /* ---- error codes ---- */
 #define B200LP_OK            0
@@ -85,6 +90,20 @@ typedef struct {
 	int32_t resident;     /* mid-size LPs (m ~ 128 ... 1500): keep A and B^-1 in the shared memory of the whole grid
 	                         (simplex_resident): 0 = auto (when they fit), -1 = never */
 	double  harris_delta; /* ratio_mode 2: feasibility tolerance of the first pass (e.g. 1e-9) */
+	int32_t algorithm;    /* 0 = primal simplex (default, everything above); 1 = dual simplex from the slack basis, for
+	                         LPs with "<=" rows of negative b (">=" constraints) and a dual feasible start (e.g. c <= 0).
+	                         One iteration:
+	                           r = argmin (x_b[i], i), lowest index on ties;
+	                           e_j = y.a_j - c_j for all n columns and, when x_b[r] < -eps, alpha_rj = rho.a_j with
+	                             rho = row r of B^-1, from the same pass over A;
+	                           min e_j < -eps -> B200LP_STATUS_NOT_DUAL_FEASIBLE; x_b[r] >= -eps -> OPTIMUM;
+	                           p = argmin (max(e_j, 0) / -alpha_rj, j) over the nonbasic columns with
+	                             alpha_rj < -pivot_tol; none -> B200LP_STATUS_INFEASIBLE;
+	                           pivot on (p, q = r) exactly like the primal loop.
+	                         iterations, pivots, trace, z and min_reduced_cost (min e_j of the last pass) keep their
+	                         primal meaning.  Single GPU, general persistent kernel at every size (simplex_dual);
+	                         needs pricing_rule = 0, ratio_mode = 0, mode = 0 and fuse_ratio <= 0, else B200LP_ERR_ARG
+	                         (checked before any device call, like algorithm outside {0, 1} and ndev > 1). */
 } b200lp_options;
 
 typedef struct {
@@ -146,14 +165,16 @@ int b200lp_solve_f32_multi(const float* A, const float* b, const float* c, int64
  *
  * Selection: the LPs run in simplex_tiny_batch (one CTA per LP, persistent grid, all of an LP in shared memory)
  * when m <= 64 (f64) / 128 (f32), A, B^-1 and the vectors of the LP with the most stored columns fit in 200 KB
- * of shared memory, pricing_rule = 0, ratio_mode != 2 and max_iter > 0.  Otherwise they run one after another on
+ * of shared memory, pricing_rule = 0, ratio_mode != 2, algorithm = 0 and max_iter > 0.  Otherwise they run one after another on
  * one engine (the single call's path without its per-call allocation), so the call accepts every shape and option
  * b200lp_solve_* accepts.  The single-engine tuning options grid_ctas, tile_shape, mode, profile, price_cols,
  * price_mode, price_tail, fuse_book2, fuse_ratio, ratio_group_rows, resident and l2_persist_mb affect only that
- * fallback; eps, max_iter, device, check_slack, pivot_tol, pricing_rule, ratio_mode and harris_delta apply to both.
+ * fallback; eps, max_iter, device, check_slack, pivot_tol, pricing_rule, ratio_mode, harris_delta and algorithm
+ * apply to both.
  *
  * Argument errors (B200LP_ERR_ARG, before any device call): batch <= 0, m <= 0, m > n, NULL A / b / c / x_b /
- * b_ixs / res, trace_cap < 0.  No device: B200LP_ERR_NO_GPU.
+ * b_ixs / res, trace_cap < 0, an algorithm the options do not allow (see b200lp_options.algorithm).  No device:
+ * B200LP_ERR_NO_GPU.
  */
 int b200lp_solve_batch_f64(const double* A, const double* b, const double* c, int64_t batch, int64_t m, int64_t n,
 		const b200lp_options* opt, double* x_b, int32_t* b_ixs, double* y,
@@ -206,7 +227,8 @@ int b200lp_download_trace(b200lp_engine* e, int32_t* trace_pq, int64_t cap, int6
 
 /* ---- per-phase entry points (unit tests, sharded multi-GPU driver) ----
  * Each runs ONE phase of the pivot as its own launch on the engine's stream and
- * waits for it.  Order within a pivot: price -> update_ftran -> ratio -> pivot_update. */
+ * waits for it.  Order within a pivot: price -> update_ftran -> ratio -> pivot_update.  These are the phases of the
+ * primal loop, whatever options.algorithm says. */
 /* pricing fused with argmin (replaces cublasSgemm + cub ArgMin, v4:289-296) */
 int b200lp_phase_price(b200lp_engine* e, int64_t* p, double* min_e);
 /* pending rank-1 update of B^-1 fused with alpha = B^-1 A[:,p] (v4:307-308 + v4:333 of the previous pivot) */

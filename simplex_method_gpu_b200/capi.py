@@ -9,6 +9,7 @@ import os
 from ._build import LIB_PATH
 
 STATUS_MAX_ITER, STATUS_OPTIMUM, STATUS_UNBOUNDED, STATUS_THETA_OVERFLOW = 0, 1, 2, 3
+STATUS_INFEASIBLE, STATUS_NOT_DUAL_FEASIBLE = 4, 5      # dual simplex (options.algorithm = 1) only
 OK, ERR_ARG, ERR_CUDA, ERR_NO_GPU, ERR_STATE = 0, -1, -2, -3, -4
 F32, F64 = 0, 1
 
@@ -38,7 +39,7 @@ class Options(C.Structure):
                 ("price_mode", C.c_int32), ("ratio_group_rows", C.c_int32), ("pivot_tol", C.c_double),
                 ("price_tail", C.c_int32), ("fuse_book2", C.c_int32), ("fuse_ratio", C.c_int32),
                 ("pricing_rule", C.c_int32), ("ratio_mode", C.c_int32), ("resident", C.c_int32),
-                ("harris_delta", C.c_double)]
+                ("harris_delta", C.c_double), ("algorithm", C.c_int32)]
 
 
 class Result(C.Structure):

@@ -85,6 +85,18 @@ bool tiny_fits(long long m, long long n, long long ns) {
 	return TinyLayout<T>(m, n, ns).bytes(m) <= (size_t)200 * 1024;
 }
 
+// options.algorithm against the rest of the options and the number of GPUs; host only, before any device call
+int check_algorithm(const b200lp_options& o, int ngpus) {
+	if (o.algorithm != 0 && o.algorithm != 1) return fail(B200LP_ERR_ARG, "algorithm must be 0 (primal) or 1 (dual)");
+	if (o.algorithm == 0) return B200LP_OK;
+	if (o.pricing_rule != 0) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) needs pricing_rule = 0");
+	if (o.ratio_mode != 0) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) needs ratio_mode = 0");
+	if (o.mode != 0) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) needs the persistent kernel (mode = 0)");
+	if (o.fuse_ratio > 0) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) has no fused ratio test (fuse_ratio > 0)");
+	if (ngpus > 1) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) runs on one GPU");
+	return B200LP_OK;
+}
+
 template <typename T>
 class Engine final : public b200lp_engine {
 	friend class MultiEngine<T>;
@@ -92,6 +104,7 @@ class Engine final : public b200lp_engine {
 public:
 	Engine(int64_t m, int64_t n, const b200lp_options& o, int rank_, int nranks_) : opt(o) {
 		std::memset(&d, 0, sizeof(d));
+		std::memset(&dd, 0, sizeof(dd));
 		std::memset(&hc, 0, sizeof(hc));
 		rank = rank_;
 		nranks = nranks_;
@@ -202,7 +215,8 @@ public:
 				(const void*)k_price<T>})
 			CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, DYN_SMEM_BYTES));
 		int occ = 0;
-		if (nranks > 1 && opt.pricing_rule == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent_sharded<T, 1, true>, NT, DYN_SMEM_BYTES));
+		if (opt.algorithm == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_dual<T, 1>, NT, UF_SMEM_BYTES));
+		else if (nranks > 1 && opt.pricing_rule == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent_sharded<T, 1, true>, NT, DYN_SMEM_BYTES));
 		else if (nranks > 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent_sharded<T, 1>, NT, DYN_SMEM_BYTES));
 		else if (opt.pricing_rule == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent<T, 1, true>, NT, DYN_SMEM_BYTES));
 		else            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent<T, 1>, NT, DYN_SMEM_BYTES));
@@ -218,6 +232,12 @@ public:
 		CU(alloc(&d.cand, (size_t)max_grid + 2));
 		CU(alloc(&d.cand2, (size_t)2 * (max_grid + 2)));
 		CU(alloc(&d.cnt, (size_t)max_grid + 2));
+		if (opt.algorithm == 1) {                         // dual simplex: nonbasic mask, rho, leaving-row candidates
+			CU(alloc(&dd.nb, (size_t)d.n));
+			CU(alloc(&dd.rho, ld));
+			CU(cudaMemsetAsync(dd.rho, 0, ld * sizeof(T), stream));
+			CU(alloc(&dd.lcand, (size_t)max_grid + 2));
+		}
 
 		// tile shape of the update+FTRAN pass: tiles are handed out dynamically, so the tallest row
 		// tile that still leaves every CTA ~100 tiles keeps the tail of the pass well under 1 %
@@ -373,6 +393,10 @@ public:
 			k_gamma_init<T><<<num_sms * 4, NT, 0, stream>>>(d);
 			launches++;
 		}
+		if (opt.algorithm == 1) {                          // dual simplex: the slack basis's nonbasic columns
+			k_nonbasic_init<<<num_sms, 256, 0, stream>>>(dd.nb, d.n, d.m);
+			launches++;
+		}
 		CU(cudaGetLastError());
 		const unsigned long long xe = hc.xepoch;    // the peer-barrier epoch outlives a reset
 		std::memset(&hc, 0, sizeof(hc));
@@ -410,6 +434,17 @@ public:
 		if (pr != 0) return pr < 0 ? pr : B200LP_OK;
 		void* args[] = {&d};
 		const void* fn;
+		if (opt.algorithm == 1) {                  // dual simplex: its own loop kernel at every size
+			void* dargs[] = {&d, &dd};
+			fn = wc == 1 ? (const void*)simplex_dual<T, 1>
+			   : wc == 2 ? (const void*)simplex_dual<T, 2>
+			   : wc == 4 ? (const void*)simplex_dual<T, 4>
+			             : (const void*)simplex_dual<T, 8>;
+			CU(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(NT), dargs, UF_SMEM_BYTES, stream));
+			launches++;
+			CU(cudaEventRecord(ev1, stream));
+			return B200LP_OK;
+		}
 		if (nranks > 1) {
 			if (!peers_mapped) return fail(B200LP_ERR_STATE, "sharded engine: peers are not mapped (ipc_import / create_multi)");
 			if (opt.pricing_rule == 1)
@@ -933,7 +968,9 @@ private:
 	// tiny LPs (one warp-wide vector row, everything fits in shared memory): the shared-memory-resident kernel.
 	// Only with the automatic grid: an explicit grid_ctas asks for the general kernel.
 	bool tiny_ok() const {
-		if (nranks != 1 || opt.grid_ctas > 0 || opt.mode != 0 || d.prof_cap > 0 || opt.pricing_rule != 0 || opt.ratio_mode == 2) return false;
+		if (nranks != 1 || opt.grid_ctas > 0 || opt.mode != 0 || d.prof_cap > 0 || opt.pricing_rule != 0 || opt.ratio_mode == 2 ||
+				opt.algorithm != 0)
+			return false;
 		return tiny_fits<T>(d.m, d.n, d.ns);
 	}
 
@@ -941,7 +978,7 @@ private:
 	// Only with the automatic configuration (an explicit grid, tile shape or pricing path asks for the general kernel).
 	bool resident_ok() const {
 		if (nranks != 1 || opt.grid_ctas > 0 || opt.mode != 0 || opt.pricing_rule != 0 || opt.ratio_mode == 2 ||
-				opt.tile_shape != 0 || opt.price_mode != 0 || opt.fuse_ratio > 0 || opt.resident < 0)
+				opt.tile_shape != 0 || opt.price_mode != 0 || opt.fuse_ratio > 0 || opt.resident < 0 || opt.algorithm != 0)
 			return false;
 		if (d.m < 128) return false;                     // a handful of CTAs: the general kernel on a small grid is as good
 		const ResLayout<T> L(d.m, d.ld, d.ns, num_sms);
@@ -1009,6 +1046,7 @@ private:
 
 	b200lp_options opt;
 	Dev<T> d;
+	DualDev<T> dd;             // dual simplex state (options.algorithm = 1)
 	Ctl hc;                    // host mirror of the control block
 	T* hA = nullptr;           // mutable aliases of the const members of d
 	T* hb = nullptr;
@@ -1265,6 +1303,7 @@ int create_engine(int64_t m, int64_t n, const b200lp_options* opt, b200lp_engine
 	if (n >= ((int64_t)1 << 31)) return fail(B200LP_ERR_ARG, "n must fit a 32-bit basis index");
 	b200lp_options o;
 	if (opt) o = *opt; else b200lp_default_options(&o);
+	if (int rc = check_algorithm(o, nranks)) return rc;
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
 		cudaGetLastError();
@@ -1285,6 +1324,7 @@ int create_multi(int64_t m, int64_t n, const b200lp_options* opt, const int32_t*
 	if (!devices || ndev < 1 || ndev > MAXR) return fail(B200LP_ERR_ARG, "need 1 <= ndev <= 8 device ordinals");
 	b200lp_options o;
 	if (opt) o = *opt; else b200lp_default_options(&o);
+	if (int rc = check_algorithm(o, ndev)) return rc;
 	if (ndev == 1) {
 		o.device = devices[0];
 		return create_engine<T>(m, n, &o, out);
@@ -1429,8 +1469,8 @@ int solve_once(const T* A, const T* b, const T* c, int64_t m, int64_t n, const b
 	return rc;
 }
 
-// Many LPs of one shape in one call (b200lp_solve_batch_*).  Tiny shapes with the Dantzig rule and a one-pass ratio
-// test run in simplex_tiny_batch (one CTA per LP, a persistent grid fed by a ticket counter); everything else runs
+// Many LPs of one shape in one call (b200lp_solve_batch_*).  Tiny shapes with the primal Dantzig rule and a one-pass
+// ratio test run in simplex_tiny_batch (one CTA per LP, a persistent grid fed by a ticket counter); everything else runs
 // the LPs one after another on one engine (upload, run, download per LP).  Either way record k and row k of every
 // output are bit-identical to b200lp_solve_* on LP k alone.
 template <typename T>
@@ -1461,7 +1501,8 @@ public:
 			for (auto& t : th) t.join();
 		}
 		const int ns_max = *std::max_element(ns.begin(), ns.end());
-		if (o.max_iter > 0 && o.pricing_rule == 0 && o.ratio_mode != 2 && tiny_fits<T>(m, n, ns_max)) return run_kernel(ns, ns_max);
+		if (o.max_iter > 0 && o.pricing_rule == 0 && o.ratio_mode != 2 && o.algorithm == 0 && tiny_fits<T>(m, n, ns_max))
+			return run_kernel(ns, ns_max);
 		return run_engine();
 	}
 
@@ -1618,6 +1659,7 @@ int solve_batch(const T* A, const T* b, const T* c, int64_t batch, int64_t m, in
 	if (opt) o = *opt; else b200lp_default_options(&o);
 	if (o.pricing_rule != 0 && o.pricing_rule != 1) return fail(B200LP_ERR_ARG, "pricing_rule must be 0 (Dantzig) or 1 (steepest edge)");
 	if (o.ratio_mode < 0 || o.ratio_mode > 2) return fail(B200LP_ERR_ARG, "ratio_mode must be 0, 1 or 2");
+	if (int rc = check_algorithm(o, 1)) return rc;
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
 		cudaGetLastError();

@@ -1474,6 +1474,208 @@ __global__ void __launch_bounds__(NT, MIN_CTAS) simplex_persistent(Dev<T> d) {
 	}
 }
 
+// ---------------------------------------------------------------- dual simplex (options.algorithm = 1)
+//
+// For LPs whose slack basis is dual feasible (every e_j = y.a_j - c_j >= 0, e.g. c <= 0) but primal infeasible
+// (some b_i < 0).  One iteration:
+//   r = argmin (x_b_i, i)                                     leaving row
+//   e_j = y.a_j - c_j and, when x_b_r < -eps, alpha_rj = rho.a_j from the same bytes of A, rho = row r of B^-1
+//       after the pending rank-1 update (rho_j = fma(E_q[r], row_q[j], B[r,j]), the update pass's own fma)
+//   min e < -eps -> NOT_DUAL_FEASIBLE;  x_b_r >= -eps -> OPTIMUM
+//   p = argmin (max(e_j, 0) / -alpha_rj, j) over the NONBASIC columns with alpha_rj < -pivot_tol; none -> INFEASIBLE
+//   basis change with q = r: the primal pivot's update + FTRAN, chunk sums of alpha, book1 and book2, unchanged.
+// The nonbasic mask is needed: with product-form rounding a basic column can get alpha_rj ~ -1e-17 and ratio 0.
+// Sums keep the primal kernel's associations (file header), both argmins are lexicographic.
+//
+// Phases and grid barriers per pivot (the primal loop has four; the two streaming passes are the same bytes):
+//   reduce the leaving-row candidates -> r;  rho gather (only when x_b_r < -eps)              | D1
+//   price_phase_dual: e_j, alpha_rj, min-e and ratio candidates per CTA                      | D2 -> statuses, p
+//   update + FTRAN of a_p                                                                     | D3
+//   alpha = chunk sums                                                                        | D4
+//   book1 (row_q, E_q, dot partials)                                                          | D5
+//   book2 (x_b, y, c_b, b_ixs), nonbasic mask, leaving-row candidates of the new x_b          | D6
+template <typename T>
+struct DualDev {
+	unsigned char* nb;        // n flags: 1 = column j is nonbasic (upload / reset: the first n - m columns)
+	T* rho;                   // ld: row r of B^-1 (padding rows zero)
+	Cand* lcand;              // one per CTA: (min x_b, row) over the CTA's rows
+};
+
+// (min x_b_i, i) over rows part*NT + tid, stride nparts*NT: the rows book2_phase updates in this thread, so it
+// runs right behind it without a barrier
+template <typename T>
+__device__ void dual_leave_cands(const Dev<T>& d, const DualDev<T>& dd, Smem& sh, int part, int nparts) {
+	double best_v = CUDART_INF;
+	long long best_i = LLONG_MAX;
+	for (long long i = (long long)part * NT + threadIdx.x; i < d.m; i += (long long)nparts * NT) {
+		const double v = (double)d.x_b[i];
+		if (cand_better(v, i, best_v, best_i)) { best_v = v; best_i = i; }
+	}
+	block_argmin(best_v, best_i, sh);
+	if (threadIdx.x == 0) { dd.lcand[part].val = best_v; dd.lcand[part].idx = best_i; }
+}
+
+// rho = row r of B^-1 with the pending rank-1 update applied on the fly (bit-identical to a flushed B^-1)
+template <typename T>
+__device__ void dual_rho_phase(const Dev<T>& d, const DualDev<T>& dd, long long r, bool pending, int part, int nparts) {
+	const T er = pending ? d.E_q[r] : T(0);
+	for (long long j = (long long)part * NT + threadIdx.x; j < d.m; j += (long long)nparts * NT) {
+		const T bj = d.B[r + j * d.ldb];
+		dd.rho[j] = pending ? fma_t(er, __ldcg(d.row_q + j), bj) : bj;
+	}
+}
+
+// e_j = y.a_j - c_j (+ alpha_rj = rho.a_j when want_alpha) for all n columns, one read of A; per CTA the
+// (min e, index) candidate -> cand[part] and the dual ratio candidate (max(e,0) / -alpha, index) over the nonbasic
+// columns with alpha < -pivot_tol -> cand2[part]
+template <typename T>
+__device__ void price_phase_dual(const Dev<T>& d, const DualDev<T>& dd, Smem& sh, bool want_alpha, int part, int nparts) {
+	const int tid = threadIdx.x;
+	double best_v = CUDART_INF, rat_v = CUDART_INF;
+	long long best_i = LLONG_MAX, rat_i = LLONG_MAX;
+	const T tol = (T)d.pivot_tol;
+	auto consider = [&](long long j, T e, T a) {
+		if (cand_better((double)e, j, best_v, best_i)) { best_v = (double)e; best_i = j; }
+		if (want_alpha && dd.nb[j] && a < -tol) {
+			const double rt = (double)((e > T(0) ? e : T(0)) / -a);
+			if (cand_better(rt, j, rat_v, rat_i)) { rat_v = rt; rat_i = j; }
+		}
+	};
+
+	const T* const vec[3] = {d.y, dd.rho, nullptr};
+	const long long c1 = d.nsl;
+	const long long nq = c1 / PRICE_NC;
+	const long long nitems = nq + (c1 - nq * PRICE_NC);
+	int buf = 0;
+	for (long long g = part; g < nitems; buf ^= 1) {
+		if (tid == 0) sh.tk = (long long)nparts + atomicAdd(&d.ctl->price_ctr, 1u);
+		const bool quad = g < nq;
+		const long long col = quad ? g * PRICE_NC : nq * PRICE_NC + (g - nq);
+		const T* base = d.A + col * d.ld;
+		if (want_alpha) {
+			if (quad) column_dots<T, PRICE_NC, 2, 2, false>(base, d.ld, d.ld, vec, sh, buf);
+			else      column_dots<T, 1, 8, 2, false>(base, d.ld, d.ld, vec, sh, buf);
+		} else {
+			if (quad) column_dots<T, PRICE_NC, 4, 1, false>(base, d.ld, d.ld, vec, sh, buf);
+			else      column_dots<T, 1, 16, 1, false>(base, d.ld, d.ld, vec, sh, buf);
+		}
+		__syncthreads();
+		g = sh.tk;
+		if (tid < (quad ? PRICE_NC : 1)) {
+			const long long j = d.col0 + col + tid;
+			const int nv = want_alpha ? 2 : 1;
+			const T e = warp_sums<T>(sh, buf, tid * nv) - d.c[j];
+			const T a = want_alpha ? warp_sums<T>(sh, buf, tid * nv + 1) : T(0);
+			consider(j, e, a);
+		}
+		__syncthreads();
+	}
+	for (long long k = d.k0 + (long long)part * NT + tid; k < d.k1; k += (long long)nparts * NT)   // unit (slack) columns
+		consider(d.ns + k, d.y[k] - d.c[d.ns + k], want_alpha ? dd.rho[k] : T(0));
+
+	block_argmin(best_v, best_i, sh);
+	block_argmin(rat_v, rat_i, sh);
+	if (tid == 0) {
+		d.cand[part].val = best_v; d.cand[part].idx = best_i;
+		d.cand2[part].val = rat_v; d.cand2[part].idx = rat_i;
+	}
+}
+
+// alpha_i = the chunk partials of row i summed left to right (ratio_phase<T, true> without its ratio test)
+template <typename T>
+__device__ void dual_alpha_phase(const Dev<T>& d, int part, int nparts) {
+	for (long long i = (long long)part * NT + threadIdx.x; i < d.m; i += (long long)nparts * NT)
+		d.alpha[i] = sum_chunk_partials(d.alpha_part + i, d.ldb, d.nchunk);
+}
+
+template <typename T, int WC>
+__global__ void __launch_bounds__(NT, MIN_CTAS) simplex_dual(Dev<T> d, DualDev<T> dd) {
+	__shared__ Smem sh;
+	extern __shared__ __align__(128) unsigned char dyn[];   // update+FTRAN staging (UF_SMEM_BYTES)
+	Ctl* ctl = d.ctl;
+	const int G = gridDim.x, me = blockIdx.x;
+	unsigned long long epoch = 0;
+
+	long long it = ctl->iter, pivots = ctl->pivots;
+	const long long it_end = ctl->it_end;
+	int pending = ctl->pending;
+	int status = 0, done = 0, aborted = 0;
+	long long p = ctl->p, q = ctl->q;
+	double min_e = ctl->min_e;
+	const long long it0 = it;
+
+	dual_leave_cands<T>(d, dd, sh, me, G);     // later ones ride behind book2
+	grid_barrier(ctl, epoch, G);
+	while (it < it_end) {
+		// ---- leaving row, rho
+		stamp(d, it - it0, 0);
+		double xr;
+		long long r;
+		reduce_cands(dd.lcand, G, xr, r, sh);
+		const bool want_alpha = xr < -d.eps;
+		if (want_alpha) {
+			dual_rho_phase<T>(d, dd, r, pending != 0, me, G);
+			grid_barrier(ctl, epoch, G);
+		}
+		// ---- column pass: reduced costs, row r of B^-1 A, both candidates
+		stamp(d, it - it0, 1);
+		price_phase_dual<T>(d, dd, sh, want_alpha, me, G);
+		stamp(d, it - it0, 2);
+		if (me == 0 && threadIdx.x == 0) ctl->abort_latched = *(volatile int*)&ctl->abort_req;
+		grid_barrier(ctl, epoch, G);
+		if (me == 0 && threadIdx.x == 0) ctl->price_ctr = 0;
+		stamp(d, it - it0, 3);
+		long long pmin, pe;
+		double rt;
+		reduce_cands(d.cand, G, min_e, pmin, sh);
+		reduce_cands(d.cand2, G, rt, pe, sh);
+		if (__ldcg(&ctl->abort_latched)) { aborted = 1; break; }
+		if (min_e < -d.eps) { status = 5; done = 1; ++it; break; }   // B200LP_STATUS_NOT_DUAL_FEASIBLE
+		if (!want_alpha) { status = 1; done = 1; ++it; break; }      // x_b >= -eps everywhere: optimum
+		if (pe == LLONG_MAX) { status = 4; done = 1; ++it; break; }  // row r is a Farkas certificate: infeasible
+		p = pe;
+		q = r;
+
+		// ---- basis change with the primal pivot's phases
+		const T* acol = p < d.ns ? d.A + p * d.ld : nullptr;
+		if (pending) update_ftran_phase<T, WC, true, true, false>(d, sh, dyn, acol, p - d.ns, pivots & 1, me, G);
+		else         update_ftran_phase<T, WC, false, true, false>(d, sh, dyn, acol, p - d.ns, pivots & 1, me, G);
+		pending = 0;
+		stamp(d, it - it0, 4);
+		grid_barrier(ctl, epoch, G);
+		if (me == 0 && threadIdx.x == 0) ctl->upd_ctr = 0;
+		dual_alpha_phase<T>(d, me, G);
+		const long long leaving = d.b_ixs[q];      // b_ixs[q] is rewritten by book2, barriers from here
+		stamp(d, it - it0, 5);
+		grid_barrier(ctl, epoch, G);
+		book1_phase<T>(d, sh, p, q, me, G);
+		stamp(d, it - it0, 6);
+		grid_barrier(ctl, epoch, G);
+		if (me == 0 && threadIdx.x == 0) {
+			if (pivots < d.trace_cap) d.trace[pivots] = make_int2((int)p, (int)q);
+			dd.nb[p] = 0;
+			dd.nb[leaving] = 1;
+		}
+		stamp(d, it - it0, 7);
+		book2_phase<T>(d, sh, p, q, me, G);
+		dual_leave_cands<T>(d, dd, sh, me, G);
+		stamp(d, it - it0, 8);
+		grid_barrier(ctl, epoch, G);
+		pending = 1;
+		++pivots;
+		++it;
+	}
+
+	if (me == 0) {
+		const double z = objective<T>(d, sh);
+		if (threadIdx.x == 0) {
+			ctl->iter = it; ctl->pivots = pivots; ctl->pending = pending;
+			ctl->status = status; ctl->done = done; ctl->aborted = aborted;
+			ctl->p = p; ctl->q = q; ctl->min_e = min_e; ctl->z = z;
+		}
+	}
+}
+
 // ---------------------------------------------------------------- tiny LPs: everything in shared memory
 //
 // Klee-Minty (m = 20, 2^20 - 1 pivots) and friends: the matrices fit in one SM's shared memory and a pivot is
@@ -2756,6 +2958,12 @@ __global__ void k_reset(Dev<T> d) {
 		d.row_q[i] = T(0);
 		if (in) d.b_ixs[i] = (int)(d.n - d.m + i);
 	}
+}
+
+// nonbasic mask of the slack basis (dual simplex): the first n - m columns are nonbasic, the last m basic
+__global__ void k_nonbasic_init(unsigned char* nb, long long n, long long m) {
+	for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (long long)gridDim.x * blockDim.x)
+		nb[j] = j < n - m ? 1 : 0;
 }
 
 __host__ __device__ __forceinline__ uint64_t mix64(uint64_t z) {

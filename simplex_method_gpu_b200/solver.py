@@ -20,11 +20,13 @@ from . import capi
 
 
 class SolveStatus(enum.IntEnum):
-    """`enum class SolveStatus` (v4:49-54)."""
+    """`enum class SolveStatus` (v4:49-54), plus the two outcomes only the dual simplex (algorithm=1) reports."""
     MaxIter = 0
     OptimumFound = 1
     Unbounded = 2
     ThetaOverflow = 3
+    Infeasible = 4           # the constraints have no solution (row r of B^-1 is a Farkas certificate)
+    NotDualFeasible = 5      # some reduced cost < -eps: the dual method cannot run from this basis
 
 
 # reference compile-time constants (v4:12, 18-19)
@@ -86,7 +88,9 @@ def _prep(A, b, c, dtype):
 def solve(A, b, c, eps: float = EPS, max_iter: int = MAX_ITER, dtype=None, device: int = 0,
           trace_cap: int | None = None, devices=None, **opts) -> Solution:
     """Drop-in for the reference's ``solve()`` (v4:219): host arrays in, host arrays out.
-    ``devices``: list of CUDA ordinals -> b200lp_solve_*_multi (B^-1 row-sharded, A column-sharded over them)."""
+    ``devices``: list of CUDA ordinals -> b200lp_solve_*_multi (B^-1 row-sharded, A column-sharded over them).
+    ``opts``: any field of b200lp_options, e.g. ``algorithm=1`` for the dual simplex (LPs with negative b and a
+    dual feasible slack basis, such as c <= 0)."""
     A, b, c, m, n, dt = _prep(A, b, c, dtype)
     L = capi.lib()
     o = capi.default_options(eps=eps, max_iter=int(max_iter), device=device, **opts)
@@ -477,6 +481,10 @@ def format_result(sol: Solution) -> str:
         out.write("Problem unbounded.\n")
     elif sol.status == SolveStatus.ThetaOverflow:
         out.write("Theta overflow.\n")
+    elif sol.status == SolveStatus.Infeasible:
+        out.write("Problem infeasible.\n")
+    elif sol.status == SolveStatus.NotDualFeasible:
+        out.write("Start not dual feasible.\n")
     else:
         out.write("MAX_ITER exceeded.\n")
     out.write("\n")
