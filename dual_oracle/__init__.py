@@ -1,10 +1,12 @@
 """TEST INFRASTRUCTURE — NOT PRODUCT CODE.
 
-ctypes front-end of the CPU reference of the dual simplex loop (``libdualoracle.so``, built in-tree with gcc by
-``build()``), the check of the engine's ``algorithm=1`` path.  Order 1 replays the engine's summation orders, so the
+ctypes front-end of the CPU reference of the dual simplex loop and of the composite method built on it
+(``libdualoracle.so``, built in-tree with gcc by ``build()``), the check of the engine's ``algorithm=1`` path with and
+without ``cost_shift=1``.  Order 1 replays the engine's summation orders, so the
 two compare bit for bit.  Only ``tests/``, ``tools/`` and ``__graft_entry__`` import it; the product path never does.
 
-Also ``gen_covering``: the synthetic dense LP negated, whose slack basis is dual feasible and primal infeasible.
+Also ``gen_covering``: the synthetic dense LP negated, whose slack basis is dual feasible and primal infeasible, and
+``gen_general``: LPs whose slack basis is neither (the composite method's inputs).
 """
 from __future__ import annotations
 
@@ -22,12 +24,12 @@ _LIB_PATH = os.path.join(_HERE, "libdualoracle.so")
 _SRCS = [os.path.join(_HERE, f) for f in ("dual_oracle.c", "dual_oracle_impl.h")] + \
         [os.path.join(_ORACLE, f) for f in ("simplex_oracle_impl.h", "simplex_oracle.h")]
 
-MAX_ITER, OPTIMUM, INFEASIBLE, NOT_DUAL_FEASIBLE = 0, 1, 4, 5
+MAX_ITER, OPTIMUM, UNBOUNDED, INFEASIBLE, NOT_DUAL_FEASIBLE = 0, 1, 2, 4, 5
 
 
 class _Result(C.Structure):
     _fields_ = [("status", C.c_int), ("iterations", C.c_long), ("pivots", C.c_long), ("z", C.c_double),
-                ("min_e", C.c_double)]
+                ("min_e", C.c_double), ("phase", C.c_int), ("shifted", C.c_long), ("phase1_pivots", C.c_long)]
 
 
 def _cc() -> str:
@@ -61,6 +63,7 @@ def lib() -> C.CDLL:
             fn = getattr(L, name)
             fn.restype = C.c_int
             fn.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_long, C.c_long, real, C.c_long, C.c_int, C.c_double,
+                           C.c_int, C.c_double,
                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_long, C.POINTER(_Result)]
         _lib = L
@@ -79,9 +82,12 @@ class DualSolution:
     y: np.ndarray
     trace_p: np.ndarray
     trace_q: np.ndarray
-    gap_p: np.ndarray            # runner-up distance of the dual ratio test (entering column)
-    gap_q: np.ndarray            # runner-up distance of the leaving-row argmin (x_b)
+    gap_p: np.ndarray            # runner-up distance of the entering column (dual ratio test; phase 2: pricing)
+    gap_q: np.ndarray            # runner-up distance of the leaving row (x_b argmin; phase 2: primal ratio test)
     Binv: np.ndarray | None = field(default=None, repr=False)
+    phase: int = 0               # composite method: 1 (ended in the dual loop) or 2 (in the primal loop)
+    shifted: int = 0             # columns the cost shift moved
+    phase1_pivots: int = 0
 
     def x(self, n: int) -> np.ndarray:
         out = np.zeros(n, dtype=self.x_b.dtype)
@@ -94,8 +100,9 @@ def _ptr(a):
 
 
 def solve(A, b, c, eps=1e-9, max_iter=100000, order=0, pivot_tol=0.0, want_Binv=False,
-          trace_cap=None) -> DualSolution:
-    """Dual simplex from the slack basis.  A: (m, n), slack block last; float32 or float64."""
+          trace_cap=None, cost_shift=0, shift_delta=0.0) -> DualSolution:
+    """Dual simplex from the slack basis; with ``cost_shift=1`` the composite method (dual loop on shifted costs, then
+    the primal loop).  A: (m, n), slack block last; float32 or float64."""
     dt = np.dtype(A.dtype)
     assert dt in (np.float32, np.float64)
     A = np.asfortranarray(A, dtype=dt)
@@ -114,12 +121,13 @@ def solve(A, b, c, eps=1e-9, max_iter=100000, order=0, pivot_tol=0.0, want_Binv=
     res = _Result()
     fn = lib().dual_solve_f64 if dt == np.float64 else lib().dual_solve_f32
     rc = fn(_ptr(A), _ptr(b), _ptr(c), m, n, eps, int(max_iter), int(order), float(pivot_tol),
+            int(cost_shift), float(shift_delta),
             _ptr(x_b), _ptr(b_ixs), _ptr(y), _ptr(Binv), _ptr(tp), _ptr(tq), _ptr(gp), _ptr(gq), cap, C.byref(res))
     if rc != 0:
         raise ValueError(f"dual_solve failed with code {rc} (m={m}, n={n})")
     k = min(res.pivots, cap)
     return DualSolution(res.status, res.iterations, res.pivots, res.z, res.min_e, x_b, b_ixs, y,
-                        tp[:k], tq[:k], gp[:k], gq[:k], Binv)
+                        tp[:k], tq[:k], gp[:k], gq[:k], Binv, res.phase, res.shifted, res.phase1_pivots)
 
 
 def gen_covering(m: int, n: int, seed: int = 1, dtype=np.float64):
@@ -133,3 +141,53 @@ def gen_covering(m: int, n: int, seed: int = 1, dtype=np.float64):
     c = -c
     c[ns:] = 0                     # +0, not -0
     return A, -b, c
+
+
+GENERAL_KINDS = ("feasible", "infeasible", "unbounded", "degenerate")
+
+
+def gen_general(m: int, n: int, seed: int = 1, kind: str = "feasible", dtype=np.float64):
+    """max c.x, A_s x <= b, x >= 0 with mixed-sign b and c: the slack basis is neither primal nor dual feasible.
+    A = [A_s, I] (m x n, n - m >= 2 structural columns), c = [c_s, 0].
+      feasible    A_s ~ U(-1, 1), b = A_s x0 + U(0.1, 1) for a known x0 ~ U(0, 1), c_s ~ U(-1, 1); the last row is
+                  sum(x) <= sum(x0) + 1, so the LP is bounded and x0 strictly feasible
+      infeasible  as feasible, with row m-2 = -(row 0) and b = -b_0 - 1, which contradicts row 0 (needs m >= 3)
+      unbounded   as feasible without the bounding row (a random row instead) and with column 0 = -U(0, 1),
+                  c_0 ~ U(0.5, 1): x_0 grows without bound
+      degenerate  integer data: A_s in {-3..3}, x0 in {0, 1, 2}, b = A_s x0 + {0, 1}, c_s in {-3..3}, every third row
+                  a copy of the row before it, bounding row as in feasible"""
+    if kind not in GENERAL_KINDS:
+        raise ValueError(f"kind must be one of {GENERAL_KINDS}")
+    ns = n - m
+    assert ns >= 2 and m >= 1
+    rng = np.random.default_rng([seed, GENERAL_KINDS.index(kind)])
+    if kind == "degenerate":
+        As = rng.integers(-3, 4, size=(m, ns)).astype(np.float64)
+        x0 = rng.integers(0, 3, size=ns).astype(np.float64)
+        for i in range(2, m - 1, 3):
+            As[i] = As[i - 1]
+        b = As @ x0 + rng.integers(0, 2, size=m)
+        for i in range(2, m - 1, 3):
+            b[i] = b[i - 1]
+        cs = rng.integers(-3, 4, size=ns).astype(np.float64)
+    else:
+        As = rng.uniform(-1.0, 1.0, size=(m, ns))
+        x0 = rng.uniform(0.0, 1.0, size=ns)
+        b = As @ x0 + rng.uniform(0.1, 1.0, size=m)
+        cs = rng.uniform(-1.0, 1.0, size=ns)
+    if kind != "unbounded":
+        As[m - 1] = 1.0
+        b[m - 1] = x0.sum() + 1.0
+    if kind == "infeasible":
+        assert m >= 3
+        As[m - 2] = -As[0]
+        b[m - 2] = -b[0] - 1.0
+    if kind == "unbounded":
+        As[:, 0] = -rng.uniform(0.0, 1.0, size=m)
+        cs[0] = rng.uniform(0.5, 1.0)
+    A = np.zeros((m, n), dtype=dtype, order="F")
+    A[:, :ns] = As
+    A[:, ns:] = np.eye(m)
+    c = np.zeros(n, dtype=dtype)
+    c[:ns] = cs
+    return A, b.astype(dtype), c

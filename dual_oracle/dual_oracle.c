@@ -1,6 +1,6 @@
 /*
  * TEST INFRASTRUCTURE — NOT PRODUCT CODE.
- * CPU reference of the dual simplex loop (see dual_oracle_impl.h).  The summation-order helpers (dot_seq,
+ * CPU reference of the dual simplex loop and of the composite method (see dual_oracle_impl.h).  The summation-order helpers (dot_seq,
  * dot_block256, dot_sliced) are the primal oracle's own, taken from oracle/simplex_oracle_impl.h unchanged.
  * Build: see __init__.py (gcc -O3 -fopenmp -ffp-contract=off, the primal oracle's flags)
  */
@@ -16,6 +16,9 @@ typedef struct {
 	long pivots;
 	double z;
 	double min_e;    /* min e_j of the last column pass */
+	int phase;       /* composite method: 1 dual loop on the shifted costs, 2 primal loop; 0 without cost_shift */
+	long shifted;    /* columns the cost shift moved */
+	long phase1_pivots;
 } dual_result;
 
 #define REAL double

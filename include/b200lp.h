@@ -104,6 +104,31 @@ typedef struct {
 	                         primal meaning.  Single GPU, general persistent kernel at every size (simplex_dual);
 	                         needs pricing_rule = 0, ratio_mode = 0, mode = 0 and fuse_ratio <= 0, else B200LP_ERR_ARG
 	                         (checked before any device call, like algorithm outside {0, 1} and ndev > 1). */
+	int32_t cost_shift;   /* 1 (with algorithm = 1): composite method for LPs whose slack basis is neither primal
+	                         feasible (some b_i < 0) nor dual feasible (some c_j > 0), e.g. max c.x with ">=" rows.
+	                         No columns are added; both phases are the existing loops.
+	                           shift: at the first run after upload / generate_dense / reset (slack basis, y = c_b),
+	                             e_j = y.a_j - c_j for every nonbasic column (the dual pricing's association); where
+	                             e_j < -eps, c'_j = y.a_j - delta_j with delta_j = shift_delta * (1 + |c_j|), else c'_j = c_j.
+	                             Slack columns are basic and never shifted.  The engine keeps the original c apart.
+	                           phase 1: the dual loop above on c' (its start is dual feasible by construction).
+	                             INFEASIBLE ends the run (feasibility does not depend on c); NOT_DUAL_FEASIBLE is only
+	                             possible through rounding drift and is reported as is.  OPTIMUM with no shifted
+	                             column ends the run: it is the plain algorithm = 1 run, status included.
+	                           hand-over (after a phase-1 OPTIMUM with a shifted column): the pending rank-1 update
+	                             is applied, c is restored, c_b[i] = c[b_ixs[i]], and y = c_b^T B^-1 when phase 1 made
+	                             a pivot (B^-1 = I otherwise and y stays).
+	                           phase 2: the primal loop (Dantzig, textbook ratio test, pivot_tol) from that basis with
+	                             the original c, in whichever primal kernel algorithm = 0 would pick.  It ends in
+	                             OPTIMUM, UNBOUNDED or MAX_ITER.
+	                         iterations, pivots and the trace run across both phases; max_iter and b200lp_run(e, k)
+	                         count the total; the phase-1 check that finds x_b >= -eps is one iteration.  A window that
+	                         ends on the phase-1 OPTIMUM performs the hand-over and reports MAX_ITER with z = c_b.x_b for
+	                         the original c.  z and min_reduced_cost are the current phase's: after a stop inside phase 1
+	                         they refer to c'.  Needs algorithm = 1 (and so everything algorithm = 1 needs), else
+	                         B200LP_ERR_ARG before any device call.  0 = off (default). */
+	double  shift_delta;  /* cost_shift: relative size of the shift (delta_j above); 0 = default 1e-7; < 0 or NaN:
+	                         B200LP_ERR_ARG */
 } b200lp_options;
 
 typedef struct {
@@ -119,7 +144,8 @@ typedef struct {
 	int64_t kernel_launches;
 } b200lp_result;
 
-/* defaults: eps 1e-4, max_iter 5 (the reference's constants), device 0, auto grid */
+/* defaults: eps 1e-4, max_iter 5 (the reference's constants), device 0, auto grid, algorithm 0, cost_shift 0 (off),
+ * shift_delta 0 (= 1e-7 when cost_shift is on) */
 void b200lp_default_options(b200lp_options* opt);
 
 /*
@@ -165,12 +191,13 @@ int b200lp_solve_f32_multi(const float* A, const float* b, const float* c, int64
  *
  * Selection: the LPs run in simplex_tiny_batch (one CTA per LP, persistent grid, all of an LP in shared memory)
  * when m <= 64 (f64) / 128 (f32), A, B^-1 and the vectors of the LP with the most stored columns fit in 200 KB
- * of shared memory, pricing_rule = 0, ratio_mode != 2, algorithm = 0 and max_iter > 0.  Otherwise they run one after another on
+ * of shared memory, pricing_rule = 0, ratio_mode != 2, algorithm = 0 and max_iter > 0 (so batches with cost_shift
+ * always take the one-engine path).  Otherwise they run one after another on
  * one engine (the single call's path without its per-call allocation), so the call accepts every shape and option
  * b200lp_solve_* accepts.  The single-engine tuning options grid_ctas, tile_shape, mode, profile, price_cols,
  * price_mode, price_tail, fuse_book2, fuse_ratio, ratio_group_rows, resident and l2_persist_mb affect only that
- * fallback; eps, max_iter, device, check_slack, pivot_tol, pricing_rule, ratio_mode, harris_delta and algorithm
- * apply to both.
+ * fallback; eps, max_iter, device, check_slack, pivot_tol, pricing_rule, ratio_mode, harris_delta, algorithm,
+ * cost_shift and shift_delta apply to both.
  *
  * Argument errors (B200LP_ERR_ARG, before any device call): batch <= 0, m <= 0, m > n, NULL A / b / c / x_b /
  * b_ixs / res, trace_cap < 0, an algorithm the options do not allow (see b200lp_options.algorithm).  No device:
@@ -214,6 +241,10 @@ int b200lp_run(b200lp_engine* e, int64_t iterations, b200lp_result* res);
 /* same, without waiting: returns after the launch; pair with b200lp_wait() */
 int b200lp_run_async(b200lp_engine* e, int64_t iterations);
 int b200lp_wait(b200lp_engine* e, b200lp_result* res);
+/* composite method (options.cost_shift = 1): phase 0 (no run since upload / generate_dense / reset), 1 (dual loop on
+ * the shifted costs) or 2 (primal loop on the original costs); shifted_columns counts the columns the shift moved,
+ * phase1_pivots the pivots of phase 1.  Any pointer may be NULL.  Engines without cost_shift report 0, 0, 0. */
+int b200lp_phase_info(b200lp_engine* e, int32_t* phase, int64_t* shifted_columns, int64_t* phase1_pivots);
 /* ask a running loop (b200lp_run_async, or b200lp_run on another thread) to stop at its next iteration boundary;
  * state stays consistent and the run can be continued.  The kernel polls one word per iteration. */
 int b200lp_abort(b200lp_engine* e);

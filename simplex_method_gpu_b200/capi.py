@@ -26,7 +26,7 @@ EXPORTS = [
     "b200lp_profile_stamps", "b200lp_profile_names", "b200lp_download_profile", "b200lp_check_basis",
     "b200lp_solve_f64_multi", "b200lp_solve_f32_multi", "b200lp_create_multi", "b200lp_abort",
     "b200lp_refactor", "b200lp_run_guarded", "b200lp_sizeof_options", "b200lp_sizeof_result",
-    "b200lp_solve_batch_f64", "b200lp_solve_batch_f32",
+    "b200lp_solve_batch_f64", "b200lp_solve_batch_f32", "b200lp_phase_info",
     # include/b200lp_io.h
     "b200lp_read_lp", "b200lp_write_lp_text", "b200lp_write_lp_binary", "b200lp_free_problem",
 ]
@@ -39,7 +39,8 @@ class Options(C.Structure):
                 ("price_mode", C.c_int32), ("ratio_group_rows", C.c_int32), ("pivot_tol", C.c_double),
                 ("price_tail", C.c_int32), ("fuse_book2", C.c_int32), ("fuse_ratio", C.c_int32),
                 ("pricing_rule", C.c_int32), ("ratio_mode", C.c_int32), ("resident", C.c_int32),
-                ("harris_delta", C.c_double), ("algorithm", C.c_int32)]
+                ("harris_delta", C.c_double), ("algorithm", C.c_int32),
+                ("cost_shift", C.c_int32), ("shift_delta", C.c_double)]
 
 
 class Result(C.Structure):
@@ -94,6 +95,7 @@ def lib() -> C.CDLL:
         "b200lp_run": (C.c_int, [vp, i64, PR]),
         "b200lp_run_async": (C.c_int, [vp, i64]),
         "b200lp_wait": (C.c_int, [vp, PR]),
+        "b200lp_phase_info": (C.c_int, [vp, C.POINTER(i32), C.POINTER(i64), C.POINTER(i64)]),
         "b200lp_download": (C.c_int, [vp, vp, vp, vp]),
         "b200lp_download_binv": (C.c_int, [vp, vp]),
         "b200lp_download_trace": (C.c_int, [vp, vp, i64, C.POINTER(i64)]),

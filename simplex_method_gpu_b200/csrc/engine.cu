@@ -64,6 +64,13 @@ struct b200lp_engine {
 	virtual int check_basis(double* xb_err, double* xb_scale) = 0;
 	virtual int abort() = 0;
 	virtual int refactor(double rel_pivot_tol, int64_t* replayed) = 0;
+	// composite method (options.cost_shift): only the single-GPU engine has phases
+	virtual int phase_info(int32_t* phase, int64_t* shifted, int64_t* phase1_pivots) {
+		if (phase) *phase = 0;
+		if (shifted) *shifted = 0;
+		if (phase1_pivots) *phase1_pivots = 0;
+		return B200LP_OK;
+	}
 	cudaStream_t stream = nullptr;
 	int rank = 0, nranks = 1;
 	int grid = 0;
@@ -94,6 +101,14 @@ int check_algorithm(const b200lp_options& o, int ngpus) {
 	if (o.mode != 0) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) needs the persistent kernel (mode = 0)");
 	if (o.fuse_ratio > 0) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) has no fused ratio test (fuse_ratio > 0)");
 	if (ngpus > 1) return fail(B200LP_ERR_ARG, "the dual simplex (algorithm = 1) runs on one GPU");
+	return B200LP_OK;
+}
+
+// options.cost_shift / shift_delta (composite method: dual phase on shifted costs, then primal); after check_algorithm
+int check_cost_shift(const b200lp_options& o) {
+	if (o.cost_shift != 0 && o.cost_shift != 1) return fail(B200LP_ERR_ARG, "cost_shift must be 0 (off) or 1 (on)");
+	if (!(o.shift_delta >= 0)) return fail(B200LP_ERR_ARG, "shift_delta must be >= 0 (0 = default) and not NaN");
+	if (o.cost_shift == 1 && o.algorithm != 1) return fail(B200LP_ERR_ARG, "cost_shift = 1 needs the dual simplex (algorithm = 1)");
 	return B200LP_OK;
 }
 
@@ -215,7 +230,13 @@ public:
 				(const void*)k_price<T>})
 			CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, DYN_SMEM_BYTES));
 		int occ = 0;
-		if (opt.algorithm == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_dual<T, 1>, NT, UF_SMEM_BYTES));
+		if (opt.algorithm == 1 && opt.cost_shift == 1) {   // phase 2 launches the primal kernel on the same grid
+			int occ2 = 0;
+			CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_dual<T, 1>, NT, UF_SMEM_BYTES));
+			CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, simplex_persistent<T, 1>, NT, DYN_SMEM_BYTES));
+			occ = std::min(occ, occ2);
+		}
+		else if (opt.algorithm == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_dual<T, 1>, NT, UF_SMEM_BYTES));
 		else if (nranks > 1 && opt.pricing_rule == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent_sharded<T, 1, true>, NT, DYN_SMEM_BYTES));
 		else if (nranks > 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent_sharded<T, 1>, NT, DYN_SMEM_BYTES));
 		else if (opt.pricing_rule == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent<T, 1, true>, NT, DYN_SMEM_BYTES));
@@ -237,6 +258,10 @@ public:
 			CU(alloc(&dd.rho, ld));
 			CU(cudaMemsetAsync(dd.rho, 0, ld * sizeof(T), stream));
 			CU(alloc(&dd.lcand, (size_t)max_grid + 2));
+		}
+		if (opt.cost_shift == 1) {                        // composite method: the original c, the shifted-column count
+			CU(alloc(&c_orig, (size_t)d.n));
+			CU(alloc(&d_shifted, 1));
 		}
 
 		// tile shape of the update+FTRAN pass: tiles are handed out dynamically, so the tallest row
@@ -335,6 +360,7 @@ public:
 		const T* b = static_cast<const T*>(bv);
 		const T* c = static_cast<const T*>(cv);
 		const long long m = d.m, n = d.n, ld = d.ld;
+		if (int rc = settle()) return rc;              // a composite run in flight may still write c (hand-over)
 		CU(cudaEventRecord(ev0, stream));
 		if (d.nsl > 0)
 			CU(cudaMemcpy2DAsync(hA, ld * sizeof(T), A, m * sizeof(T), m * sizeof(T), (size_t)d.nsl,
@@ -342,6 +368,7 @@ public:
 		CU(cudaMemsetAsync(hb, 0, ld * sizeof(T), stream));
 		CU(cudaMemcpyAsync(hb, b, m * sizeof(T), cudaMemcpyHostToDevice, stream));
 		CU(cudaMemcpyAsync(hcst, c, n * sizeof(T), cudaMemcpyHostToDevice, stream));
+		c_shifted = false;
 		if (ld > m && d.nsl > 0) {
 			k_zero_pad<T><<<num_sms * 4, 256, 0, stream>>>(hA, m, ld, d.nsl);
 			launches++;
@@ -365,10 +392,12 @@ public:
 
 	int generate_dense(uint64_t seed) override {
 		CU(cudaSetDevice(opt.device));
+		if (int rc = settle()) return rc;
 		CU(set_columns(d.n - d.m));
 		k_generate_dense<T><<<num_sms * 8, 256, 0, stream>>>(hA, hb, hcst, d.m, d.n, d.ns, d.ld, seed, d.col0, d.nsl);
 		launches++;
 		CU(cudaGetLastError());
+		c_shifted = false;
 		have_data = true;
 		return reset();
 	}
@@ -387,6 +416,12 @@ public:
 		CU(cudaSetDevice(opt.device));
 		if (int rc = settle()) return rc;
 		CU(ensure_B());
+		if (c_shifted) {                                   // composite method: back to the original c before c_b, y
+			CU(cudaMemcpyAsync(hcst, c_orig, (size_t)d.n * sizeof(T), cudaMemcpyDeviceToDevice, stream));
+			c_shifted = false;
+		}
+		phase = 0;
+		shifted_cols = ph1_pivots = 0;
 		k_reset<T><<<num_sms * 8, 256, 0, stream>>>(d);
 		launches++;
 		if (opt.pricing_rule == 1) {                       // steepest edge: the weights start over with the slack basis
@@ -426,6 +461,9 @@ public:
 		if (d.prof_cap > 0) CU(cudaMemsetAsync(d.prof, 0, (size_t)d.prof_cap * NSTAMP * sizeof(unsigned long long), stream));
 		prof_iter0 = hc.iter;
 		CU(cudaEventRecord(ev0, stream));
+		if (opt.cost_shift == 1 && phase == 0) {           // first run from the slack basis: shift, then phase 1
+			if (int rc = shift_costs()) return rc;
+		}
 		return 0;
 	}
 
@@ -434,7 +472,7 @@ public:
 		if (pr != 0) return pr < 0 ? pr : B200LP_OK;
 		void* args[] = {&d};
 		const void* fn;
-		if (opt.algorithm == 1) {                  // dual simplex: its own loop kernel at every size
+		if (!primal_loop()) {                      // dual simplex: its own loop kernel at every size
 			void* dargs[] = {&d, &dd};
 			fn = wc == 1 ? (const void*)simplex_dual<T, 1>
 			   : wc == 2 ? (const void*)simplex_dual<T, 2>
@@ -478,6 +516,7 @@ public:
 	int abort() override {
 		CU(cudaSetDevice(opt.device));
 		if (!in_flight) return B200LP_OK;
+		abort_asked = true;                        // also keeps wait() from starting phase 2 of the composite method
 		if (!abort_stream) CU(cudaStreamCreateWithFlags(&abort_stream, cudaStreamNonBlocking));
 		int* one = reinterpret_cast<int*>(static_cast<unsigned char*>(pinned) + sizeof(Ctl));
 		*one = 1;
@@ -501,6 +540,26 @@ public:
 		}
 		in_flight = false;
 		if (hc.bad) return fail(B200LP_ERR_CUDA, "sharded engine: a peer GPU did not answer within 20 s (the engine must be destroyed)");
+		ms_run += ms;
+		if (opt.cost_shift == 1 && phase == 1) {
+			if (shift_unread) {
+				unsigned long long k = 0;
+				CU(cudaMemcpy(&k, d_shifted, sizeof(k), cudaMemcpyDeviceToHost));
+				shifted_cols = (int64_t)k;
+				shift_unread = false;
+			}
+			ph1_pivots = hc.pivots;
+			// phase 1 at the optimum of c': hand over to the primal loop, and run it with what is left of the budget
+			if (hc.done && hc.status == B200LP_STATUS_OPTIMUM && shifted_cols > 0) {
+				if (int rc = hand_over()) return rc;
+				if (abort_asked) was_aborted = true;
+				else if (hc.it_end > hc.iter) {
+					if (int rc = run_async(hc.it_end - hc.iter)) return rc;
+					return wait(res);
+				}
+			}
+		}
+		abort_asked = false;
 		if (res) {
 			std::memset(res, 0, sizeof(*res));
 			res->status = hc.status;
@@ -509,10 +568,18 @@ public:
 			res->pivots = hc.pivots;
 			res->z = hc.z;
 			res->min_reduced_cost = hc.min_e;
-			res->ms_solve = ms;
+			res->ms_solve = ms_run;
 			res->ms_upload = ms_upload;
 			res->kernel_launches = launches;
 		}
+		ms_run = 0;
+		return B200LP_OK;
+	}
+
+	int phase_info(int32_t* ph, int64_t* shifted, int64_t* phase1_pivots) override {
+		if (ph) *ph = phase;
+		if (shifted) *shifted = shifted_cols;
+		if (phase1_pivots) *phase1_pivots = ph1_pivots;
 		return B200LP_OK;
 	}
 
@@ -965,11 +1032,60 @@ private:
 		launches++;
 	}
 
+	// the primal loop runs: algorithm = 0, or phase 2 of the composite method (algorithm = 1, cost_shift = 1)
+	bool primal_loop() const { return opt.algorithm == 0 || phase == 2; }
+
+	// composite method, first run from the slack basis: keep the original c, shift the nonbasic columns with
+	// e_j < -eps (k_cost_shift), then phase 1 (the dual loop) prices with c'.  The count is read by wait().
+	int shift_costs() {
+		CU(cudaMemcpyAsync(c_orig, hcst, (size_t)d.n * sizeof(T), cudaMemcpyDeviceToDevice, stream));
+		CU(cudaMemsetAsync(d_shifted, 0, sizeof(unsigned long long), stream));
+		const T delta = (T)(opt.shift_delta > 0 ? opt.shift_delta : 1e-7);
+		k_cost_shift<T><<<num_sms * 4, NT, 0, stream>>>(d, hcst, dd.nb, delta, d_shifted);
+		launches++;
+		CU(cudaGetLastError());
+		c_shifted = true;
+		shift_unread = true;
+		phase = 1;
+		return B200LP_OK;
+	}
+
+	// composite method, after a phase-1 OPTIMUM with shifted columns: flush the pending rank-1 update (as check_basis
+	// and refactor do), restore c, c_b = c[b_ixs], y = c_b^T B^-1 (as refactor does; B^-1 = I and y unchanged when
+	// phase 1 made no pivot), z for the original c, and a control block as a primal window boundary leaves it:
+	// nothing pending, not done.  simplex_persistent / _tiny / _resident read iter, pivots, pending, p, q and min_e at
+	// entry; p and q are used only with a pending book2 (fuse_book2 never carries one across launches) or the
+	// steepest-edge recurrence (pricing_rule = 0 here).
+	int hand_over() {
+		if (hc.pending) { launch_update_ftran(true, false, 0); hc.pending = 0; }
+		CU(cudaMemcpyAsync(hcst, c_orig, (size_t)d.n * sizeof(T), cudaMemcpyDeviceToDevice, stream));
+		c_shifted = false;
+		k_gather_cb<T><<<num_sms, 256, 0, stream>>>(d.c_b, d.c, d.b_ixs, d.m);
+		launches++;
+		if (hc.pivots > 0) {
+			k_btran_vec<T><<<num_sms * 2, NT, 0, stream>>>(d, d.c_b, d.acol);
+			k_copy<T><<<num_sms, 256, 0, stream>>>(d.y, d.acol, d.m);
+			launches += 2;
+		}
+		k_objective<T><<<1, NT, 0, stream>>>(d);
+		launches++;
+		CU(cudaGetLastError());
+		CU(cudaStreamSynchronize(stream));
+		Ctl t;
+		CU(cudaMemcpy(&t, d.ctl, sizeof(Ctl), cudaMemcpyDeviceToHost));
+		hc.z = t.z;
+		hc.done = 0;
+		hc.status = B200LP_STATUS_MAX_ITER;
+		phase = 2;
+		CU(push_ctl());
+		return B200LP_OK;
+	}
+
 	// tiny LPs (one warp-wide vector row, everything fits in shared memory): the shared-memory-resident kernel.
 	// Only with the automatic grid: an explicit grid_ctas asks for the general kernel.
 	bool tiny_ok() const {
 		if (nranks != 1 || opt.grid_ctas > 0 || opt.mode != 0 || d.prof_cap > 0 || opt.pricing_rule != 0 || opt.ratio_mode == 2 ||
-				opt.algorithm != 0)
+				!primal_loop())
 			return false;
 		return tiny_fits<T>(d.m, d.n, d.ns);
 	}
@@ -978,7 +1094,7 @@ private:
 	// Only with the automatic configuration (an explicit grid, tile shape or pricing path asks for the general kernel).
 	bool resident_ok() const {
 		if (nranks != 1 || opt.grid_ctas > 0 || opt.mode != 0 || opt.pricing_rule != 0 || opt.ratio_mode == 2 ||
-				opt.tile_shape != 0 || opt.price_mode != 0 || opt.fuse_ratio > 0 || opt.resident < 0 || opt.algorithm != 0)
+				opt.tile_shape != 0 || opt.price_mode != 0 || opt.fuse_ratio > 0 || opt.resident < 0 || !primal_loop())
 			return false;
 		if (d.m < 128) return false;                     // a handful of CTAs: the general kernel on a small grid is as good
 		const ResLayout<T> L(d.m, d.ld, d.ns, num_sms);
@@ -1047,6 +1163,14 @@ private:
 	b200lp_options opt;
 	Dev<T> d;
 	DualDev<T> dd;             // dual simplex state (options.algorithm = 1)
+	T* c_orig = nullptr;       // composite method (options.cost_shift): the original c while d.c holds c'
+	unsigned long long* d_shifted = nullptr;   // columns k_cost_shift moved
+	int phase = 0;             // composite method: 0 not started, 1 dual loop on c', 2 primal loop on c
+	int64_t shifted_cols = 0, ph1_pivots = 0;
+	bool c_shifted = false;    // d.c holds c' (c_orig the original)
+	bool shift_unread = false; // d_shifted not read back yet
+	std::atomic<bool> abort_asked{false};
+	double ms_run = 0;         // device time of the phases of the current run
 	Ctl hc;                    // host mirror of the control block
 	T* hA = nullptr;           // mutable aliases of the const members of d
 	T* hb = nullptr;
@@ -1304,6 +1428,7 @@ int create_engine(int64_t m, int64_t n, const b200lp_options* opt, b200lp_engine
 	b200lp_options o;
 	if (opt) o = *opt; else b200lp_default_options(&o);
 	if (int rc = check_algorithm(o, nranks)) return rc;
+	if (int rc = check_cost_shift(o)) return rc;
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
 		cudaGetLastError();
@@ -1325,6 +1450,7 @@ int create_multi(int64_t m, int64_t n, const b200lp_options* opt, const int32_t*
 	b200lp_options o;
 	if (opt) o = *opt; else b200lp_default_options(&o);
 	if (int rc = check_algorithm(o, ndev)) return rc;
+	if (int rc = check_cost_shift(o)) return rc;
 	if (ndev == 1) {
 		o.device = devices[0];
 		return create_engine<T>(m, n, &o, out);
@@ -1471,7 +1597,8 @@ int solve_once(const T* A, const T* b, const T* c, int64_t m, int64_t n, const b
 
 // Many LPs of one shape in one call (b200lp_solve_batch_*).  Tiny shapes with the primal Dantzig rule and a one-pass
 // ratio test run in simplex_tiny_batch (one CTA per LP, a persistent grid fed by a ticket counter); everything else runs
-// the LPs one after another on one engine (upload, run, download per LP).  Either way record k and row k of every
+// the LPs one after another on one engine (upload, run, download per LP), among them every batch of the dual or the
+// composite method (cost_shift needs algorithm = 1, the batch kernel algorithm = 0).  Either way record k and row k of every
 // output are bit-identical to b200lp_solve_* on LP k alone.
 template <typename T>
 class BatchCall {
@@ -1660,6 +1787,7 @@ int solve_batch(const T* A, const T* b, const T* c, int64_t batch, int64_t m, in
 	if (o.pricing_rule != 0 && o.pricing_rule != 1) return fail(B200LP_ERR_ARG, "pricing_rule must be 0 (Dantzig) or 1 (steepest edge)");
 	if (o.ratio_mode < 0 || o.ratio_mode > 2) return fail(B200LP_ERR_ARG, "ratio_mode must be 0, 1 or 2");
 	if (int rc = check_algorithm(o, 1)) return rc;
+	if (int rc = check_cost_shift(o)) return rc;
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
 		cudaGetLastError();
@@ -1834,6 +1962,10 @@ int b200lp_run(b200lp_engine* e, int64_t iterations, b200lp_result* res) {
 }
 int b200lp_run_async(b200lp_engine* e, int64_t iterations) { NEED(e); return e->run_async(iterations); }
 int b200lp_wait(b200lp_engine* e, b200lp_result* res) { NEED(e); return e->wait(res); }
+int b200lp_phase_info(b200lp_engine* e, int32_t* phase, int64_t* shifted_columns, int64_t* phase1_pivots) {
+	NEED(e);
+	return e->phase_info(phase, shifted_columns, phase1_pivots);
+}
 int b200lp_abort(b200lp_engine* e) { NEED(e); return e->abort(); }
 int b200lp_refactor(b200lp_engine* e, double rel_pivot_tol, int64_t* replayed) { NEED(e); return e->refactor(rel_pivot_tol, replayed); }
 

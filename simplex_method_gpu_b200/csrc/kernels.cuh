@@ -2966,6 +2966,44 @@ __global__ void k_nonbasic_init(unsigned char* nb, long long n, long long m) {
 		nb[j] = j < n - m ? 1 : 0;
 }
 
+__device__ __forceinline__ double mul_rn_t(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn_t(float a, float b) { return __fmul_rn(a, b); }
+
+// Cost shift of the composite method (options.cost_shift), from the slack basis: for every stored nonbasic column,
+// s = y.a_j in the pricing association and e_j = s - c_j (the dual pricing's own numbers); where e_j < -eps,
+// c_j <- s - delta (1 + |c_j|) (a product rounded on its own, never fused into the subtraction) and the column is
+// counted.  Unit (slack) columns are basic at the start and are not visited.  c is rewritten in place: the caller
+// keeps the original.
+template <typename T>
+__global__ void __launch_bounds__(NT) k_cost_shift(Dev<T> d, T* c, const unsigned char* nb, T delta,
+		unsigned long long* shifted) {
+	__shared__ Smem sh;
+	const T* const v3[3] = {d.y, nullptr, nullptr};
+	int buf = 0;
+	for (long long col = blockIdx.x; col < d.nsl; col += gridDim.x, buf ^= 1) {
+		const long long j = d.col0 + col;
+		if (!nb[j]) continue;                         // the same for the whole CTA
+		column_dots<T, 1, 16, 1, false>(d.A + col * d.ld, d.ld, d.ld, v3, sh, buf);
+		__syncthreads();
+		if (threadIdx.x == 0) {
+			const T s = warp_sums<T>(sh, buf, 0);
+			const T cj = c[j];
+			if ((double)(s - cj) < -d.eps) {
+				c[j] = s - mul_rn_t(delta, T(1) + (cj < T(0) ? -cj : cj));
+				atomicAdd(shifted, 1ull);
+			}
+		}
+		__syncthreads();
+	}
+}
+
+// c_b[i] = c[b_ixs[i]] (hand-over of the composite method: the basis costs of the original c)
+template <typename T>
+__global__ void k_gather_cb(T* c_b, const T* c, const int* b_ixs, long long m) {
+	for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (long long)gridDim.x * blockDim.x)
+		c_b[i] = c[b_ixs[i]];
+}
+
 __host__ __device__ __forceinline__ uint64_t mix64(uint64_t z) {
 	z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ULL;
 	z = (z ^ (z >> 27)) * 0x94D049BB133111EBULL;

@@ -1,7 +1,10 @@
 // CLI with the driver contract of the reference's main() (src/v4_cub_reduction.cu:384-474):
 //   solver.out <lp.txt | lp.b200lp> [--f64] [--eps E] [--max-iter N] [--device D] [--gpus N | --devices a,b,..] [--dual]
+//              [--cost-shift]
 // --dual: the dual simplex from the slack basis (options.algorithm = 1; negative b, dual feasible start), which can
 // also print "Problem infeasible." or "Start not dual feasible.".
+// --cost-shift (with --dual): the composite method (options.cost_shift = 1) for LPs with both negative b and positive c:
+// the dual loop on shifted costs, then the primal loop on the original ones.
 // Same input text format (v4:401-420; parsed by b200lp_read_lp, which also accepts the binary twin), same stdout: one "# Iteration k" line per
 // iteration (v4:287), the result block (v4:426-445) and the timing block
 // (v4:456-471, same labels and number format).  Defaults reproduce the reference's
@@ -129,6 +132,7 @@ int main(int argc, char* argv[]) {
 		else if (!std::strcmp(argv[i], "--max-iter") && i + 1 < argc) opt.max_iter = std::atoll(argv[++i]);
 		else if (!std::strcmp(argv[i], "--device") && i + 1 < argc) opt.device = std::atoi(argv[++i]);
 		else if (!std::strcmp(argv[i], "--dual")) opt.algorithm = 1;
+		else if (!std::strcmp(argv[i], "--cost-shift")) opt.cost_shift = 1;
 		else if (!std::strcmp(argv[i], "--gpus") && i + 1 < argc) {
 			g_devices.clear();
 			for (int k = 0, nk = std::atoi(argv[++i]); k < nk; ++k) g_devices.push_back(k);

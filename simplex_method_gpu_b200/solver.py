@@ -90,7 +90,8 @@ def solve(A, b, c, eps: float = EPS, max_iter: int = MAX_ITER, dtype=None, devic
     """Drop-in for the reference's ``solve()`` (v4:219): host arrays in, host arrays out.
     ``devices``: list of CUDA ordinals -> b200lp_solve_*_multi (B^-1 row-sharded, A column-sharded over them).
     ``opts``: any field of b200lp_options, e.g. ``algorithm=1`` for the dual simplex (LPs with negative b and a
-    dual feasible slack basis, such as c <= 0)."""
+    dual feasible slack basis, such as c <= 0), ``algorithm=1, cost_shift=1`` for the composite method (LPs with
+    negative b and positive c: the dual loop on shifted costs, then the primal loop)."""
     A, b, c, m, n, dt = _prep(A, b, c, dtype)
     L = capi.lib()
     o = capi.default_options(eps=eps, max_iter=int(max_iter), device=device, **opts)
@@ -255,6 +256,13 @@ class Engine:
         res = capi.Result()
         capi.check(self._L.b200lp_wait(self._h, C.byref(res)))
         return self._result(res)
+
+    def phase_info(self) -> dict:
+        """Composite method (cost_shift=1): phase 0 (not started), 1 (dual loop on the shifted costs) or 2 (primal loop
+        on the original costs), the number of shifted columns and the pivots of phase 1 (b200lp_phase_info)."""
+        ph, k, p1 = C.c_int32(0), C.c_int64(0), C.c_int64(0)
+        capi.check(self._L.b200lp_phase_info(self._h, C.byref(ph), C.byref(k), C.byref(p1)))
+        return {"phase": ph.value, "shifted_columns": k.value, "phase1_pivots": p1.value}
 
     def refactor(self, rel_pivot_tol: float = 0.0) -> int:
         """Rebuild B^-1, x_b and y from the current basis (b200lp_refactor); returns the number of replayed pivots."""
