@@ -101,7 +101,8 @@ typedef struct {
 	                             alpha_rj < -pivot_tol; none -> B200LP_STATUS_INFEASIBLE;
 	                           pivot on (p, q = r) exactly like the primal loop.
 	                         iterations, pivots, trace, z and min_reduced_cost (min e_j of the last pass) keep their
-	                         primal meaning.  Single GPU, general persistent kernel at every size (simplex_dual);
+	                         primal meaning.  Single GPU, general persistent kernel at every size (simplex_dual;
+	                         tiny batches of b200lp_solve_batch_*: simplex_tiny_batch_dual, the same bits);
 	                         needs pricing_rule = 0, ratio_mode = 0, mode = 0 and fuse_ratio <= 0, else B200LP_ERR_ARG
 	                         (checked before any device call, like algorithm outside {0, 1} and ndev > 1). */
 	int32_t cost_shift;   /* 1 (with algorithm = 1): composite method for LPs whose slack basis is neither primal
@@ -189,10 +190,12 @@ int b200lp_solve_f32_multi(const float* A, const float* b, const float* c, int64
  * Contract: record k and row k of every output are bit-identical to b200lp_solve_f64 / _f32 called on LP k alone
  * with the same options (y: to b200lp_download after such a run).
  *
- * Selection: the LPs run in simplex_tiny_batch (one CTA per LP, persistent grid, all of an LP in shared memory)
- * when m <= 64 (f64) / 128 (f32), A, B^-1 and the vectors of the LP with the most stored columns fit in 200 KB
- * of shared memory, pricing_rule = 0, ratio_mode != 2, algorithm = 0 and max_iter > 0 (so batches with cost_shift
- * always take the one-engine path).  Otherwise they run one after another on
+ * Selection: the LPs run in one kernel, one CTA per LP on a persistent grid with all of an LP in shared memory,
+ * when m <= 64 (f64) / 128 (f32), A, B^-1 and the vectors of the LP with the most stored columns fit in 200 KB of
+ * shared memory and max_iter > 0: simplex_tiny_batch for algorithm = 0 with pricing_rule = 0 and ratio_mode != 2,
+ * simplex_tiny_batch_dual for algorithm = 1 with or without cost_shift (the dual's layout adds one byte per
+ * column, its nonbasic mask, to the 200 KB test).  That kernel runs the single call's sequence per LP: the cost shift,
+ * the dual loop, the hand-over and the primal loop.  Otherwise the LPs run one after another on
  * one engine (the single call's path without its per-call allocation), so the call accepts every shape and option
  * b200lp_solve_* accepts.  The single-engine tuning options grid_ctas, tile_shape, mode, profile, price_cols,
  * price_mode, price_tail, fuse_book2, fuse_ratio, ratio_group_rows, resident and l2_persist_mb affect only that

@@ -92,6 +92,14 @@ bool tiny_fits(long long m, long long n, long long ns) {
 	return TinyLayout<T>(m, n, ns).bytes(m) <= (size_t)200 * 1024;
 }
 
+// the same question for simplex_tiny_batch_dual (dual simplex / composite batches), whose layout adds the nonbasic
+// mask: a shape can fit tiny_fits and not this
+template <typename T>
+bool tiny_dual_fits(long long m, long long n, long long ns) {
+	if (m > TinyLayout<T>::LD) return false;
+	return TinyDualLayout<T>(m, n, ns).bytes(m, n) <= (size_t)200 * 1024;
+}
+
 // options.algorithm against the rest of the options and the number of GPUs; host only, before any device call
 int check_algorithm(const b200lp_options& o, int ngpus) {
 	if (o.algorithm != 0 && o.algorithm != 1) return fail(B200LP_ERR_ARG, "algorithm must be 0 (primal) or 1 (dual)");
@@ -1595,11 +1603,11 @@ int solve_once(const T* A, const T* b, const T* c, int64_t m, int64_t n, const b
 	return rc;
 }
 
-// Many LPs of one shape in one call (b200lp_solve_batch_*).  Tiny shapes with the primal Dantzig rule and a one-pass
-// ratio test run in simplex_tiny_batch (one CTA per LP, a persistent grid fed by a ticket counter); everything else runs
-// the LPs one after another on one engine (upload, run, download per LP), among them every batch of the dual or the
-// composite method (cost_shift needs algorithm = 1, the batch kernel algorithm = 0).  Either way record k and row k of every
-// output are bit-identical to b200lp_solve_* on LP k alone.
+// Many LPs of one shape in one call (b200lp_solve_batch_*).  Tiny shapes run in one kernel, one CTA per LP on a
+// persistent grid fed by a ticket counter: simplex_tiny_batch for the primal Dantzig rule with a one-pass ratio test,
+// simplex_tiny_batch_dual for the dual simplex and the composite method (algorithm = 1, with or without cost_shift).
+// Everything else, and max_iter <= 0, runs the LPs one after another on one engine (upload, run, download per LP).
+// Either way record k and row k of every output are bit-identical to b200lp_solve_* on LP k alone.
 template <typename T>
 class BatchCall {
 public:
@@ -1628,6 +1636,8 @@ public:
 			for (auto& t : th) t.join();
 		}
 		const int ns_max = *std::max_element(ns.begin(), ns.end());
+		if (o.max_iter > 0 && o.algorithm == 1 && tiny_dual_fits<T>(m, n, ns_max))   // check_algorithm: Dantzig, textbook ratio
+			return run_kernel(ns, ns_max);
 		if (o.max_iter > 0 && o.pricing_rule == 0 && o.ratio_mode != 2 && o.algorithm == 0 && tiny_fits<T>(m, n, ns_max))
 			return run_kernel(ns, ns_max);
 		return run_engine();
@@ -1686,13 +1696,18 @@ private:
 		bt.pivot_tol = sizeof(T) == 4 ? (double)(float)o.pivot_tol : o.pivot_tol;
 		bt.ratio_mode = o.ratio_mode;
 		bt.x_b = dx; bt.y = dy; bt.b_ixs = dbix; bt.trace = dtr; bt.trace_cap = trace_cap; bt.rec = drec; bt.ticket = dticket;
-		const size_t smem = TinyLayout<T>(m, n, ns_max).bytes(m);
-		CU(cudaFuncSetAttribute(simplex_tiny_batch<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+		bt.cost_shift = o.cost_shift;
+		bt.delta = (T)(o.shift_delta > 0 ? o.shift_delta : 1e-7);                // as Engine::shift_costs does
+		const bool dual = o.algorithm == 1;
+		const void* fn = dual ? (const void*)simplex_tiny_batch_dual<T> : (const void*)simplex_tiny_batch<T>;
+		const size_t smem = dual ? TinyDualLayout<T>(m, n, ns_max).bytes(m, n) : TinyLayout<T>(m, n, ns_max).bytes(m);
+		CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 		int occ = 0;
-		CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_tiny_batch<T>, NT, smem));
-		if (occ < 1) return fail(B200LP_ERR_CUDA, "simplex_tiny_batch does not fit on an SM");
+		CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, NT, smem));
+		if (occ < 1) return fail(B200LP_ERR_CUDA, "the tiny batch kernel does not fit on an SM");
 		const int grid = (int)std::min<int64_t>(batch, (int64_t)occ * prop.multiProcessorCount);
-		simplex_tiny_batch<T><<<grid, NT, smem, stream>>>(bt);
+		if (dual) simplex_tiny_batch_dual<T><<<grid, NT, smem, stream>>>(bt);
+		else      simplex_tiny_batch<T><<<grid, NT, smem, stream>>>(bt);
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(ev[2], stream));
 

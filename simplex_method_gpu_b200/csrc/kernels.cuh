@@ -216,6 +216,9 @@ template <> struct Mem<float> {
 
 __device__ __forceinline__ double fma_t(double a, double b, double c) { return fma(a, b, c); }
 __device__ __forceinline__ float fma_t(float a, float b, float c) { return fmaf(a, b, c); }
+// a product rounded on its own (never contracted into an fma)
+__device__ __forceinline__ double mul_rn_t(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn_t(float a, float b) { return __fmul_rn(a, b); }
 
 template <typename T>
 __device__ __forceinline__ T warp_butterfly_sum(T s) {
@@ -1721,6 +1724,114 @@ struct TinyLP {
 		  m(m_), n(n_), ns(ns_) {}
 };
 
+// The pricing dot of the tiny kernels: the column's 32 vectors are the lanes of one warp (av, yv: this lane's
+// vector of the column and of y), the association of the general kernel's pricing dot.  Valid in every lane.
+template <typename T>
+__device__ __forceinline__ T tiny_dot(const typename VecT<T>::V& av, const typename VecT<T>::V& yv) {
+	using M = Mem<T>;
+	T s = fma_t(M::get(av, 0), M::get(yv, 0), T(0));
+#pragma unroll
+	for (int v = 1; v < VecT<T>::N; ++v) s = s + fma_t(M::get(av, v), M::get(yv, v), T(0));
+	s = warp_butterfly_sum(s);
+	return s + T(0);                               // + the seven empty warp sums of the general kernel
+}
+
+// Pending rank-1 update fused with the FTRAN of column p (v4:333 + v4:307-308): alpha = B^-1 a_p after
+// B^-1 += E_q (x) row_q when `pending`.  Shared by the primal and the dual loop; ends with a barrier.
+template <typename T>
+__device__ __forceinline__ void tiny_update_ftran(const TinyLP<T>& s, long long p, int pending) {
+	using V = typename VecT<T>::V;
+	using M = Mem<T>;
+	constexpr int VN = VecT<T>::N;
+	constexpr int LD = 32 * VN;
+	T *sA = s.A, *sB = s.B, *sal = s.alpha, *sE = s.E_q, *srq = s.row_q, *spart = s.part;
+	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	const int m = s.m, ns = s.ns;
+	{
+		const int j0 = warp * SUBW;                // this warp's 32-column sub-block
+		T acc[VN];
+		V Ev = *reinterpret_cast<const V*>(sE + lane * VN);
+#pragma unroll
+		for (int v = 0; v < VN; ++v) acc[v] = T(0);
+		const int jend = j0 + SUBW < m ? j0 + SUBW : m;
+		for (int j = j0; j < jend; ++j) {
+			V x = *reinterpret_cast<const V*>(sB + (long long)j * LD + lane * VN);
+			const T a = p < ns ? sA[(long long)p * LD + j] : (j == (int)(p - ns) ? T(1) : T(0));
+			if (pending) {
+				const T r = srq[j];
+#pragma unroll
+				for (int v = 0; v < VN; ++v) M::set(x, v, fma_t(M::get(Ev, v), r, M::get(x, v)));
+				*reinterpret_cast<V*>(sB + (long long)j * LD + lane * VN) = x;
+			}
+#pragma unroll
+			for (int v = 0; v < VN; ++v) acc[v] = fma_t(M::get(x, v), a, acc[v]);
+		}
+#pragma unroll
+		for (int v = 0; v < VN; ++v) spart[(warp * 32 + lane) * VN + v] = acc[v];
+	}
+	__syncthreads();
+	if (warp == 0) {
+		T t[NWARP][VN];
+#pragma unroll
+		for (int c = 0; c < NWARP; ++c)
+#pragma unroll
+			for (int v = 0; v < VN; ++v) t[c][v] = spart[(c * 32 + lane) * VN + v];
+#pragma unroll
+		for (int w = 1; w < NWARP; w <<= 1)
+#pragma unroll
+			for (int c = 0; c + w < NWARP; c += 2 * w)
+#pragma unroll
+				for (int v = 0; v < VN; ++v) t[c][v] = t[c][v] + t[c + w][v];
+#pragma unroll
+		for (int v = 0; v < VN; ++v) sal[lane * VN + v] = t[0][v];
+	}
+	__syncthreads();
+}
+
+// The basis change on (p, q) (v4:331-356: book1 and book2 of the general kernel, one 256-element slice): row_q, E_q,
+// x_b, y, c_b[q], b_ixs[q] and the trace entry of pivot `pivots`.  Needs alpha = B^-1 a_p; leaves the rank-1 update
+// pending.  Shared by the primal and the dual loop; ends with a barrier.
+template <typename T>
+__device__ __forceinline__ void tiny_pivot(const TinyLP<T>& s, Smem& sh, long long p, long long q, int2* trace,
+		long long trace_cap, long long pivots) {
+	constexpr int LD = 32 * VecT<T>::N;
+	T *sB = s.B, *sy = s.y, *sx = s.x_b, *scb = s.c_b, *sal = s.alpha, *sE = s.E_q, *srq = s.row_q, *sb = s.b, *sc = s.c;
+	int* sbix = s.b_ixs;
+	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	const int m = s.m;
+	const T alpha_q = sal[q];
+	const T c_p = sc[p];
+	T t1 = T(0), t2 = T(0), eq = T(0), rq = T(0);
+	const int i = tid;
+	if (i < m) {
+		rq = sB[(long long)i * LD + q];
+		eq = (i != q) ? (-sal[i] / alpha_q) : (T)(1.0 / (double)alpha_q - 1.0);
+		T cb = scb[i];
+		if (i == q) { sh.bc_v = (double)cb; cb = c_p; }
+		t1 = fma_t(rq, sb[i], T(0));
+		t2 = fma_t(cb, eq, T(0));
+	}
+	t1 = warp_butterfly_sum(t1);
+	t2 = warp_butterfly_sum(t2);
+	__syncthreads();
+	if (lane == 0) { sh.dsum[0][warp] = (double)t1; sh.dsum[1][warp] = (double)t2; }
+	if (i < LD) { srq[i] = i < m ? rq : T(0); sE[i] = i < m ? eq : T(0); }
+	__syncthreads();
+	T sxv = T(0), syv = T(0);
+#pragma unroll
+	for (int w = 0; w < NWARP; ++w) { sxv = sxv + (T)sh.dsum[0][w]; syv = syv + (T)sh.dsum[1][w]; }
+	sxv = T(0) + sxv;                              // book2 of the general kernel starts its slice sum from 0
+	syv = T(0) + syv;
+	syv += c_p - (T)sh.bc_v;
+	if (i < m) {
+		sx[i] = fma_t(sxv, eq, sx[i]);
+		sy[i] = fma_t(syv, rq, sy[i]);
+		if (i == q) { scb[i] = c_p; sbix[i] = (int)p; }
+	}
+	if (tid == 0 && pivots < trace_cap) trace[pivots] = make_int2((int)p, (int)q);
+	__syncthreads();
+}
+
 // The pivot loop of the tiny kernels (simplex_tiny, simplex_tiny_batch): iterations [it, it_end) on the LP in
 // shared memory, the scalar state in registers of every thread.  Leaves after the last iteration or at
 // optimum / unbounded (status, done set, the final iteration counted like the general kernel does).
@@ -1729,12 +1840,9 @@ __device__ __forceinline__ void tiny_pivots(const TinyLP<T>& s, Smem& sh, double
 		int2* trace, long long trace_cap, long long& it, const long long it_end, long long& pivots, int& pending,
 		int& status, int& done, long long& p, long long& q, double& min_e) {
 	using V = typename VecT<T>::V;
-	using M = Mem<T>;
 	constexpr int VN = VecT<T>::N;
 	constexpr int LD = 32 * VN;
-	T *sA = s.A, *sB = s.B, *sy = s.y, *sx = s.x_b, *scb = s.c_b, *sal = s.alpha, *sE = s.E_q, *srq = s.row_q,
-	  *sb = s.b, *spart = s.part, *sc = s.c;
-	int* sbix = s.b_ixs;
+	T *sA = s.A, *sy = s.y, *sx = s.x_b, *sal = s.alpha, *sc = s.c;
 	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 	const int m = s.m, n = s.n, ns = s.ns;
 	while (it < it_end) {
@@ -1744,12 +1852,7 @@ __device__ __forceinline__ void tiny_pivots(const TinyLP<T>& s, Smem& sh, double
 		const V yv = *reinterpret_cast<const V*>(sy + lane * VN);
 		for (int col = warp; col < ns; col += NWARP) {
 			const V av = *reinterpret_cast<const V*>(sA + (long long)col * LD + lane * VN);
-			T s = fma_t(M::get(av, 0), M::get(yv, 0), T(0));
-#pragma unroll
-			for (int v = 1; v < VN; ++v) s = s + fma_t(M::get(av, v), M::get(yv, v), T(0));
-			s = warp_butterfly_sum(s);
-			s = s + T(0);                              // + the seven empty warp sums of the general kernel
-			const double e = (double)(s - sc[col]);
+			const double e = (double)(tiny_dot<T>(av, yv) - sc[col]);
 			if (lane == 0 && cand_better(e, col, best_v, best_i)) { best_v = e; best_i = col; }
 		}
 		for (int k = tid; k < n - ns; k += NT) {       // unit (slack) columns
@@ -1761,47 +1864,8 @@ __device__ __forceinline__ void tiny_pivots(const TinyLP<T>& s, Smem& sh, double
 		p = best_i;
 		if (min_e >= -eps) { status = 1; done = 1; ++it; break; }
 
-		// ---- pending rank-1 update fused with the FTRAN of column p (v4:333 + v4:307-308)
-		{
-			const int j0 = warp * SUBW;                // this warp's 32-column sub-block
-			T acc[VN];
-			V Ev = *reinterpret_cast<const V*>(sE + lane * VN);
-#pragma unroll
-			for (int v = 0; v < VN; ++v) acc[v] = T(0);
-			const int jend = j0 + SUBW < m ? j0 + SUBW : m;
-			for (int j = j0; j < jend; ++j) {
-				V x = *reinterpret_cast<const V*>(sB + (long long)j * LD + lane * VN);
-				const T a = p < ns ? sA[(long long)p * LD + j] : (j == (int)(p - ns) ? T(1) : T(0));
-				if (pending) {
-					const T r = srq[j];
-#pragma unroll
-					for (int v = 0; v < VN; ++v) M::set(x, v, fma_t(M::get(Ev, v), r, M::get(x, v)));
-					*reinterpret_cast<V*>(sB + (long long)j * LD + lane * VN) = x;
-				}
-#pragma unroll
-				for (int v = 0; v < VN; ++v) acc[v] = fma_t(M::get(x, v), a, acc[v]);
-			}
-#pragma unroll
-			for (int v = 0; v < VN; ++v) spart[(warp * 32 + lane) * VN + v] = acc[v];
-		}
+		tiny_update_ftran(s, p, pending);
 		pending = 0;
-		__syncthreads();
-		if (warp == 0) {
-			T t[NWARP][VN];
-#pragma unroll
-			for (int c = 0; c < NWARP; ++c)
-#pragma unroll
-				for (int v = 0; v < VN; ++v) t[c][v] = spart[(c * 32 + lane) * VN + v];
-#pragma unroll
-			for (int w = 1; w < NWARP; w <<= 1)
-#pragma unroll
-				for (int c = 0; c + w < NWARP; c += 2 * w)
-#pragma unroll
-					for (int v = 0; v < VN; ++v) t[c][v] = t[c][v] + t[c + w][v];
-#pragma unroll
-			for (int v = 0; v < VN; ++v) sal[lane * VN + v] = t[0][v];
-		}
-		__syncthreads();
 
 		// ---- ratio test (v4:311-325)
 		best_v = CUDART_INF;
@@ -1827,41 +1891,83 @@ __device__ __forceinline__ void tiny_pivots(const TinyLP<T>& s, Smem& sh, double
 		for (int w = 0; w < NWARP; ++w) elig += sh.red_c[w];
 		if (elig == 0) { status = 2; done = 1; ++it; break; }
 
-		// ---- pivot (v4:331-356): one 256-element slice
-		const T alpha_q = sal[q];
-		const T c_p = sc[p];
-		T t1 = T(0), t2 = T(0), eq = T(0), rq = T(0);
-		const int i = tid;
-		if (i < m) {
-			rq = sB[(long long)i * LD + q];
-			eq = (i != q) ? (-sal[i] / alpha_q) : (T)(1.0 / (double)alpha_q - 1.0);
-			T cb = scb[i];
-			if (i == q) { sh.bc_v = (double)cb; cb = c_p; }
-			t1 = fma_t(rq, sb[i], T(0));
-			t2 = fma_t(cb, eq, T(0));
-		}
-		t1 = warp_butterfly_sum(t1);
-		t2 = warp_butterfly_sum(t2);
-		__syncthreads();
-		if (lane == 0) { sh.dsum[0][warp] = (double)t1; sh.dsum[1][warp] = (double)t2; }
-		if (i < LD) { srq[i] = i < m ? rq : T(0); sE[i] = i < m ? eq : T(0); }
-		__syncthreads();
-		T sxv = T(0), syv = T(0);
-#pragma unroll
-		for (int w = 0; w < NWARP; ++w) { sxv = sxv + (T)sh.dsum[0][w]; syv = syv + (T)sh.dsum[1][w]; }
-		sxv = T(0) + sxv;                              // book2 of the general kernel starts its slice sum from 0
-		syv = T(0) + syv;
-		syv += c_p - (T)sh.bc_v;
-		if (i < m) {
-			sx[i] = fma_t(sxv, eq, sx[i]);
-			sy[i] = fma_t(syv, rq, sy[i]);
-			if (i == q) { scb[i] = c_p; sbix[i] = (int)p; }
-		}
-		if (tid == 0 && pivots < trace_cap) trace[pivots] = make_int2((int)p, (int)q);
+		tiny_pivot(s, sh, p, q, trace, trace_cap, pivots);
 		pending = 1;
 		++pivots;
 		++it;
-		__syncthreads();
+	}
+}
+
+// The dual loop of the tiny batch kernel (simplex_tiny_batch_dual): simplex_dual's iteration (see above it) on one LP
+// in shared memory, with the same numbers in the same order:
+//   r = argmin (x_b_i, i) as double;  rho = row r of B^-1 after the pending update (dual_rho_phase's fma), held in
+//   alpha, which is dead until this iteration's FTRAN;  e_j and alpha_rj with the pricing dot (tiny_dot), unit
+//   columns y_k - c_j and rho_k (price_phase_dual);  the statuses in simplex_dual's order;  the pivot on (p, q = r)
+//   through the primal loop's own update+FTRAN and pivot blocks.  nb: the nonbasic mask (n bytes).
+template <typename T>
+__device__ __forceinline__ void tiny_dual_pivots(const TinyLP<T>& s, unsigned char* nb, Smem& sh, double eps,
+		double pivot_tol, int2* trace, long long trace_cap, long long& it, const long long it_end, long long& pivots,
+		int& pending, int& status, int& done, long long& p, long long& q, double& min_e) {
+	using V = typename VecT<T>::V;
+	constexpr int VN = VecT<T>::N;
+	constexpr int LD = 32 * VN;
+	T *sA = s.A, *sB = s.B, *sy = s.y, *sx = s.x_b, *rho = s.alpha, *sc = s.c;
+	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	const int m = s.m, n = s.n, ns = s.ns;
+	const T tol = (T)pivot_tol;
+	while (it < it_end) {
+		// ---- leaving row, rho
+		double xr = CUDART_INF;
+		long long r = LLONG_MAX;
+		for (int i = tid; i < m; i += NT)
+			if (cand_better((double)sx[i], i, xr, r)) { xr = (double)sx[i]; r = i; }
+		block_argmin(xr, r, sh);
+		const bool want_alpha = xr < -eps;
+		if (want_alpha) {
+			if (tid < LD) {
+				const T bj = tid < m ? sB[r + (long long)tid * LD] : T(0);    // padding rows +0, as in DualDev::rho
+				rho[tid] = pending && tid < m ? fma_t(s.E_q[r], s.row_q[tid], bj) : bj;
+			}
+			__syncthreads();
+		}
+
+		// ---- column pass: reduced costs, row r of B^-1 A, both candidates
+		double best_v = CUDART_INF, rat_v = CUDART_INF;
+		long long best_i = LLONG_MAX, rat_i = LLONG_MAX;
+		auto consider = [&](int j, T e, T a) {
+			if (cand_better((double)e, j, best_v, best_i)) { best_v = (double)e; best_i = j; }
+			if (want_alpha && nb[j] && a < -tol) {
+				const double rt = (double)((e > T(0) ? e : T(0)) / -a);
+				if (cand_better(rt, j, rat_v, rat_i)) { rat_v = rt; rat_i = j; }
+			}
+		};
+		const V yv = *reinterpret_cast<const V*>(sy + lane * VN);
+		const V rv = *reinterpret_cast<const V*>(rho + lane * VN);
+		for (int col = warp; col < ns; col += NWARP) {
+			const V av = *reinterpret_cast<const V*>(sA + (long long)col * LD + lane * VN);
+			const T e = tiny_dot<T>(av, yv) - sc[col];
+			const T a = want_alpha ? tiny_dot<T>(av, rv) : T(0);
+			if (lane == 0) consider(col, e, a);
+		}
+		for (int k = tid; k < n - ns; k += NT)          // unit (slack) columns
+			consider(ns + k, sy[k] - sc[ns + k], want_alpha ? rho[k] : T(0));
+		block_argmin(best_v, best_i, sh);
+		block_argmin(rat_v, rat_i, sh);
+		min_e = best_v;
+		if (min_e < -eps) { status = 5; done = 1; ++it; break; }        // B200LP_STATUS_NOT_DUAL_FEASIBLE
+		if (!want_alpha) { status = 1; done = 1; ++it; break; }         // x_b >= -eps everywhere: optimum
+		if (rat_i == LLONG_MAX) { status = 4; done = 1; ++it; break; }  // row r is a Farkas certificate: infeasible
+		p = rat_i;
+		q = r;
+
+		// ---- basis change with the primal loop's blocks
+		if (tid == 0) { nb[p] = 0; nb[s.b_ixs[q]] = 1; }   // b_ixs[q] before tiny_pivot rewrites it
+		tiny_update_ftran(s, p, pending);
+		pending = 0;
+		tiny_pivot(s, sh, p, q, trace, trace_cap, pivots);
+		pending = 1;
+		++pivots;
+		++it;
 	}
 }
 
@@ -1965,11 +2071,59 @@ struct TinyBatch {
 	long long trace_cap;
 	TinyBatchRec* rec;        // batch
 	unsigned long long* ticket; // next LP to hand out (zeroed by the host before the launch)
+	int cost_shift;           // simplex_tiny_batch_dual: 1 = composite method (options.cost_shift)
+	T delta;                  // its shift (options.shift_delta, 0 -> 1e-7, rounded to T as Engine does)
 };
+
+// state in: LP k's slack basis in shared memory, as k_reset leaves it for simplex_tiny, padding rows +0
+template <typename T>
+__device__ __forceinline__ void tiny_batch_load(const TinyBatch<T>& bt, long long k, const TinyLP<T>& s) {
+	constexpr int LD = TinyLayout<T>::LD;
+	const int tid = threadIdx.x;
+	const int m = s.m, n = s.n, ns = s.ns;
+	const T* Ak = bt.A + (size_t)k * (size_t)m * (size_t)n;
+	const T* bk = bt.b + (size_t)k * m;
+	const T* ck = bt.c + (size_t)k * n;
+	for (long long e = tid; e < (long long)LD * ns; e += NT) {
+		const int i = (int)(e % LD);
+		s.A[e] = i < m ? Ak[(e / LD) * m + i] : T(0);
+	}
+	for (long long e = tid; e < (long long)LD * m; e += NT) s.B[e] = e % LD == e / LD ? T(1) : T(0);
+	for (int i = tid; i < LD; i += NT) {
+		const bool in = i < m;
+		const T cb = in ? ck[n - m + i] : T(0);
+		const T bi = in ? bk[i] : T(0);
+		s.y[i] = cb; s.c_b[i] = cb; s.x_b[i] = bi; s.b[i] = bi;
+		s.alpha[i] = T(0); s.E_q[i] = T(0); s.row_q[i] = T(0);
+	}
+	for (int j = tid; j < n; j += NT) s.c[j] = ck[j];
+	for (int i = tid; i < m; i += NT) s.b_ixs[i] = n - m + i;
+}
+
+// state out: LP k's rows of x_b, b_ixs (and y), and its record with z = c_b . x_b; ends with the barrier after
+// which the next LP may overwrite shared memory
+template <typename T>
+__device__ __forceinline__ void tiny_batch_store(const TinyBatch<T>& bt, long long k, const TinyLP<T>& s, Smem& sh,
+		long long it, long long pivots, double min_e, int status) {
+	const int tid = threadIdx.x;
+	const int m = s.m;
+	__syncthreads();
+	for (int i = tid; i < m; i += NT) {
+		bt.x_b[(size_t)k * m + i] = s.x_b[i];
+		bt.b_ixs[(size_t)k * m + i] = s.b_ixs[i];
+		if (bt.y) bt.y[(size_t)k * m + i] = s.y[i];
+	}
+	const T z = tiny_objective(s.c_b, s.x_b, m, sh);
+	if (tid == 0) {
+		TinyBatchRec r;
+		r.iterations = it; r.pivots = pivots; r.z = (double)z; r.min_e = min_e; r.status = status; r.pad = 0;
+		bt.rec[k] = r;
+	}
+	__syncthreads();                               // shared memory (ticket, LP) is reused by the next LP
+}
 
 template <typename T>
 __global__ void __launch_bounds__(NT, TINY_BATCH_MIN_CTAS) simplex_tiny_batch(TinyBatch<T> bt) {
-	constexpr int LD = TinyLayout<T>::LD;
 	__shared__ Smem sh;
 	__shared__ long long s_k;
 	extern __shared__ __align__(128) unsigned char dynraw[];
@@ -1984,25 +2138,7 @@ __global__ void __launch_bounds__(NT, TINY_BATCH_MIN_CTAS) simplex_tiny_batch(Ti
 		const int ns = bt.ns[k];
 		const TinyLayout<T> L(m, n, ns);
 		const TinyLP<T> s(S, L, m, n, ns);
-		const T* Ak = bt.A + (size_t)k * (size_t)m * (size_t)n;
-		const T* bk = bt.b + (size_t)k * m;
-		const T* ck = bt.c + (size_t)k * n;
-
-		// ---- state in: the slack basis of k_reset, padding rows +0
-		for (long long e = tid; e < (long long)LD * ns; e += NT) {
-			const int i = (int)(e % LD);
-			s.A[e] = i < m ? Ak[(e / LD) * m + i] : T(0);
-		}
-		for (long long e = tid; e < (long long)LD * m; e += NT) s.B[e] = e % LD == e / LD ? T(1) : T(0);
-		for (int i = tid; i < LD; i += NT) {
-			const bool in = i < m;
-			const T cb = in ? ck[n - m + i] : T(0);
-			const T bi = in ? bk[i] : T(0);
-			s.y[i] = cb; s.c_b[i] = cb; s.x_b[i] = bi; s.b[i] = bi;
-			s.alpha[i] = T(0); s.E_q[i] = T(0); s.row_q[i] = T(0);
-		}
-		for (int j = tid; j < n; j += NT) s.c[j] = ck[j];
-		for (int i = tid; i < m; i += NT) s.b_ixs[i] = n - m + i;
+		tiny_batch_load(bt, k, s);
 		long long it = 0, pivots = 0, p = 0, q = 0;
 		int pending = 0, status = 0, done = 0;
 		double min_e = 0;
@@ -2011,21 +2147,99 @@ __global__ void __launch_bounds__(NT, TINY_BATCH_MIN_CTAS) simplex_tiny_batch(Ti
 		int2* tr = bt.trace ? bt.trace + (size_t)k * bt.trace_cap : nullptr;
 		tiny_pivots(s, sh, bt.eps, bt.pivot_tol, bt.ratio_mode, tr, tr ? bt.trace_cap : 0, it, bt.it_end, pivots, pending,
 			status, done, p, q, min_e);
+		tiny_batch_store(bt, k, s, sh, it, pivots, min_e, status);
+	}
+}
 
-		// ---- state out
+// Shared memory of simplex_tiny_batch_dual: TinyLayout (rho lives in alpha) and the nonbasic mask after b_ixs.
+template <typename T>
+struct TinyDualLayout : TinyLayout<T> {
+	__host__ __device__ TinyDualLayout(long long m, long long n, long long ns) : TinyLayout<T>(m, n, ns) {}
+	__host__ __device__ size_t nb(long long m) const { return (size_t)this->end * sizeof(T) + (size_t)m * sizeof(int); }
+	__host__ __device__ size_t bytes(long long m, long long n) const { return TinyLayout<T>::bytes(m) + (size_t)n; }
+};
+
+// The dual simplex (options.algorithm = 1) and the composite method (cost_shift = 1) on many tiny LPs: the grid,
+// tickets, state in and state out of simplex_tiny_batch, and per LP the single call's sequence in one CTA:
+//   cost_shift: k_cost_shift from the slack basis (y = c_b) over the stored nonbasic columns j < n - m, s = y.a_j
+//     in the pricing association, c_j <- s - mul_rn(delta, 1 + |c_j|) where (double)(s - c_j) < -eps
+//   phase 1: tiny_dual_pivots (simplex_dual) from the mask of k_nonbasic_init
+//   after a phase-1 OPTIMUM with a shifted column, Engine::hand_over: flush the pending update (the update block's
+//     fma), c from the caller's c, c_b = c[b_ixs], y_j = c_b.B^-1[:, j] (k_btran_vec's pricing association) when
+//     phase 1 pivoted, status MAX_ITER; then phase 2: tiny_pivots with the rest of max_iter.  z is c_b . x_b of
+//     whatever basis the LP stops in, which after a budget ending on the phase-1 optimum is hand_over's k_objective.
+template <typename T>
+__global__ void __launch_bounds__(NT, TINY_BATCH_MIN_CTAS) simplex_tiny_batch_dual(TinyBatch<T> bt) {
+	using V = typename VecT<T>::V;
+	constexpr int VN = VecT<T>::N;
+	constexpr int LD = TinyLayout<T>::LD;
+	__shared__ Smem sh;
+	__shared__ long long s_k;
+	extern __shared__ __align__(128) unsigned char dynraw[];
+	T* S = reinterpret_cast<T*>(dynraw);
+	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	const int m = (int)bt.m, n = (int)bt.n;
+	for (;;) {
+		if (tid == 0) s_k = (long long)atomicAdd(bt.ticket, 1ULL);
 		__syncthreads();
-		for (int i = tid; i < m; i += NT) {
-			bt.x_b[(size_t)k * m + i] = s.x_b[i];
-			bt.b_ixs[(size_t)k * m + i] = s.b_ixs[i];
-			if (bt.y) bt.y[(size_t)k * m + i] = s.y[i];
+		const long long k = s_k;
+		if (k >= bt.batch) break;
+		const int ns = bt.ns[k];
+		const TinyDualLayout<T> L(m, n, ns);
+		const TinyLP<T> s(S, L, m, n, ns);
+		unsigned char* nb = dynraw + L.nb(m);
+		tiny_batch_load(bt, k, s);
+		for (int j = tid; j < n; j += NT) nb[j] = j < n - m ? 1 : 0;
+		long long it = 0, pivots = 0, p = 0, q = 0;
+		int pending = 0, status = 0, done = 0;
+		double min_e = 0;
+		__syncthreads();
+
+		int shifted = 0;
+		if (bt.cost_shift) {
+			const V yv = *reinterpret_cast<const V*>(s.y + lane * VN);
+			for (int col = warp; col < n - m; col += NWARP) {
+				const T sd = tiny_dot<T>(*reinterpret_cast<const V*>(s.A + (long long)col * LD + lane * VN), yv);
+				if (lane == 0) {
+					const T cj = s.c[col];
+					if ((double)(sd - cj) < -bt.eps) {
+						s.c[col] = sd - mul_rn_t(bt.delta, T(1) + (cj < T(0) ? -cj : cj));
+						shifted = 1;
+					}
+				}
+			}
+			shifted = __syncthreads_or(shifted);
 		}
-		const T z = tiny_objective(s.c_b, s.x_b, m, sh);
-		if (tid == 0) {
-			TinyBatchRec r;
-			r.iterations = it; r.pivots = pivots; r.z = (double)z; r.min_e = min_e; r.status = status; r.pad = 0;
-			bt.rec[k] = r;
+
+		int2* tr = bt.trace ? bt.trace + (size_t)k * bt.trace_cap : nullptr;
+		tiny_dual_pivots(s, nb, sh, bt.eps, bt.pivot_tol, tr, tr ? bt.trace_cap : 0, it, bt.it_end, pivots, pending,
+			status, done, p, q, min_e);
+
+		if (shifted && done && status == 1) {          // hand-over to the primal loop
+			if (pending) {
+				for (long long e = tid; e < (long long)LD * m; e += NT)
+					s.B[e] = fma_t(s.E_q[e % LD], s.row_q[e / LD], s.B[e]);
+				pending = 0;
+			}
+			const T* ck = bt.c + (size_t)k * n;
+			for (int j = tid; j < n; j += NT) s.c[j] = ck[j];
+			__syncthreads();
+			for (int i = tid; i < m; i += NT) s.c_b[i] = s.c[s.b_ixs[i]];
+			__syncthreads();
+			if (pivots > 0) {
+				const V cv = *reinterpret_cast<const V*>(s.c_b + lane * VN);
+				for (int col = warp; col < m; col += NWARP) {
+					const T yj = tiny_dot<T>(*reinterpret_cast<const V*>(s.B + (long long)col * LD + lane * VN), cv);
+					if (lane == 0) s.y[col] = yj;
+				}
+				__syncthreads();
+			}
+			status = 0;                                // B200LP_STATUS_MAX_ITER
+			done = 0;
+			tiny_pivots(s, sh, bt.eps, bt.pivot_tol, bt.ratio_mode, tr, tr ? bt.trace_cap : 0, it, bt.it_end, pivots,
+				pending, status, done, p, q, min_e);
 		}
-		__syncthreads();                               // shared memory (ticket, LP) is reused by the next LP
+		tiny_batch_store(bt, k, s, sh, it, pivots, min_e, status);
 	}
 }
 
@@ -2965,9 +3179,6 @@ __global__ void k_nonbasic_init(unsigned char* nb, long long n, long long m) {
 	for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (long long)gridDim.x * blockDim.x)
 		nb[j] = j < n - m ? 1 : 0;
 }
-
-__device__ __forceinline__ double mul_rn_t(double a, double b) { return __dmul_rn(a, b); }
-__device__ __forceinline__ float mul_rn_t(float a, float b) { return __fmul_rn(a, b); }
 
 // Cost shift of the composite method (options.cost_shift), from the slack basis: for every stored nonbasic column,
 // s = y.a_j in the pricing association and e_j = s - c_j (the dual pricing's own numbers); where e_j < -eps,
