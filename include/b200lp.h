@@ -248,6 +248,16 @@ int b200lp_wait(b200lp_engine* e, b200lp_result* res);
  * the shifted costs) or 2 (primal loop on the original costs); shifted_columns counts the columns the shift moved,
  * phase1_pivots the pivots of phase 1.  Any pointer may be NULL.  Engines without cost_shift report 0, 0, 0. */
 int b200lp_phase_info(b200lp_engine* e, int32_t* phase, int64_t* shifted_columns, int64_t* phase1_pivots);
+/* touched columns of B^-1: from the slack basis only the columns of the rows that have left the basis (K) differ
+ * from e_j, so the single-GPU persistent kernel's update + FTRAN pass (and the steepest-edge BTRAN) can stream K's
+ * columns alone, with the same bits.  k = 0: auto (m >= 4096 and |K| <= m / 8, the default), -1: off (every pass streams
+ * all of B^-1), > 0: while |K| <= k.  Applies from the next run.  Never used with the fused ratio test, on sharded
+ * engines (B200LP_ERR_STATE), for m > 262144, for stored columns with an inf or NaN, and after a non-finite pivot
+ * row or alpha until the next reset / refactor.  k < -1: B200LP_ERR_ARG. */
+int b200lp_set_binv_sparse(b200lp_engine* e, int32_t k);
+/* the touched-column state since the last reset / refactor: columns of B^-1 that may differ from e_j, and how many
+ * update + FTRAN passes of the persistent kernel streamed only those.  Sharded engines report 0, 0. */
+int b200lp_binv_info(b200lp_engine* e, int64_t* touched, int64_t* sparse_passes);
 /* ask a running loop (b200lp_run_async, or b200lp_run on another thread) to stop at its next iteration boundary;
  * state stays consistent and the run can be continued.  The kernel polls one word per iteration. */
 int b200lp_abort(b200lp_engine* e);
@@ -271,7 +281,8 @@ int b200lp_phase_update_ftran(b200lp_engine* e, int64_t p);
 int b200lp_phase_ratio(b200lp_engine* e, int64_t* q, int64_t* eligible);
 /* row extract, E_q, c_b/b_ixs bookkeeping, x_b and y updates (v4:331-332, 339-356) */
 int b200lp_phase_pivot_update(b200lp_engine* e, int64_t p, int64_t q);
-/* device vectors for inspection: which = 0 alpha, 1 E_q, 2 row_q, 3 x_b, 4 y, 5 c_b (length m) */
+/* device vectors for inspection: which = 0 alpha, 1 E_q, 2 row_q, 3 x_b, 4 y, 5 c_b (length m); steepest edge
+ * (pricing_rule = 1) only: 6 v = B^-T alpha of the last pivot (length m), 7 the weights gamma (length n) */
 int b200lp_download_vector(b200lp_engine* e, int32_t which, void* out);
 
 /* ---- sharded engine: one process per GPU of one NVSwitch box (SURVEY.md 8(e)) ----

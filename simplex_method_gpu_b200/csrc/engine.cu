@@ -64,6 +64,13 @@ struct b200lp_engine {
 	virtual int check_basis(double* xb_err, double* xb_scale) = 0;
 	virtual int abort() = 0;
 	virtual int refactor(double rel_pivot_tol, int64_t* replayed) = 0;
+	// touched-column passes (b200lp_set_binv_sparse): single-GPU engine only
+	virtual int set_binv_sparse(int32_t) { return fail(B200LP_ERR_STATE, "binv_sparse: sharded engines stream all of B^-1"); }
+	virtual int binv_info(int64_t* touched, int64_t* sparse_passes) {
+		if (touched) *touched = 0;
+		if (sparse_passes) *sparse_passes = 0;
+		return B200LP_OK;
+	}
 	// composite method (options.cost_shift): only the single-GPU engine has phases
 	virtual int phase_info(int32_t* phase, int64_t* shifted, int64_t* phase1_pivots) {
 		if (phase) *phase = 0;
@@ -184,6 +191,13 @@ public:
 		d.c = hcst;
 		CU(alloc(&d.alpha_part, (size_t)d.nchunk * (size_t)d.ldb));
 		CU(alloc(&d.dpart, (size_t)3 * d.nslice));
+		d.kmask = nullptr;
+		if (nranks == 1) {                  // touched columns of B^-1 (the sharded loop streams all of its rows)
+			CU(alloc(&d.kmask, (size_t)d.nchunk * (CHUNK / SUBW)));
+			CU(cudaMemsetAsync(d.kmask, 0, (size_t)d.nchunk * (CHUNK / SUBW) * sizeof(unsigned int), stream));
+		}
+		CU(alloc(&d_nonfinite, 1));
+		set_kmax();
 		d.pricing_rule = opt.pricing_rule;
 		if (opt.pricing_rule == 1) {
 			if (opt.mode != 0) return fail(B200LP_ERR_ARG, "steepest-edge pricing needs the persistent kernel (mode = 0)");
@@ -235,6 +249,10 @@ public:
 				(const void*)simplex_persistent_sharded<T, 4, true>, (const void*)simplex_persistent_sharded<T, 8, true>,
 				(const void*)simplex_persistent<T, 1, true>, (const void*)simplex_persistent<T, 2, true>,
 				(const void*)simplex_persistent<T, 4, true>, (const void*)simplex_persistent<T, 8, true>,
+				(const void*)simplex_persistent<T, 1, false, true>, (const void*)simplex_persistent<T, 2, false, true>,
+				(const void*)simplex_persistent<T, 4, false, true>, (const void*)simplex_persistent<T, 8, false, true>,
+				(const void*)simplex_persistent<T, 1, true, true>, (const void*)simplex_persistent<T, 2, true, true>,
+				(const void*)simplex_persistent<T, 4, true, true>, (const void*)simplex_persistent<T, 8, true, true>,
 				(const void*)k_price<T>})
 			CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, DYN_SMEM_BYTES));
 		int occ = 0;
@@ -249,6 +267,12 @@ public:
 		else if (nranks > 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent_sharded<T, 1>, NT, DYN_SMEM_BYTES));
 		else if (opt.pricing_rule == 1) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent<T, 1, true>, NT, DYN_SMEM_BYTES));
 		else            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, simplex_persistent<T, 1>, NT, DYN_SMEM_BYTES));
+		if (nranks == 1 && (opt.algorithm == 0 || opt.cost_shift == 1)) {   // the touched-column variant shares the grid
+			int occk = 0;
+			CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occk, opt.pricing_rule == 1 ? simplex_persistent<T, 1, true, true>
+				: simplex_persistent<T, 1, false, true>, NT, DYN_SMEM_BYTES));
+			occ = std::min(occ, occk);
+		}
 		if (occ < 1) return fail(B200LP_ERR_CUDA, "persistent kernel does not fit on an SM");
 		max_grid = occ * num_sms;
 		const double work = (double)d.ld * (double)d.n / nranks;
@@ -381,6 +405,11 @@ public:
 			k_zero_pad<T><<<num_sms * 4, 256, 0, stream>>>(hA, m, ld, d.nsl);
 			launches++;
 		}
+		if (d.kmask) {                  // only the touched-column passes need to know
+			CU(cudaMemsetAsync(d_nonfinite, 0, sizeof(int), stream));
+			k_flag_nonfinite<T><<<num_sms * 4, 256, 0, stream>>>(hA, (long long)ld * d.nsl, d_nonfinite);
+			launches++;
+		}
 		CU(cudaEventRecord(ev1, stream));
 		CU(ensure_B());                 // while the copies are on the wire
 		return B200LP_OK;
@@ -392,6 +421,10 @@ public:
 		int rc = reset();
 		if (rc) return rc;
 		CU(cudaStreamSynchronize(stream));
+		int nf = 0;
+		if (d.kmask) CU(cudaMemcpy(&nf, d_nonfinite, sizeof(int), cudaMemcpyDeviceToHost));
+		a_nonfinite = nf != 0;
+		set_kmax();
 		float ms = 0;
 		CU(cudaEventElapsedTime(&ms, ev0, ev1));
 		ms_upload = ms;
@@ -407,6 +440,8 @@ public:
 		CU(cudaGetLastError());
 		c_shifted = false;
 		have_data = true;
+		a_nonfinite = false;
+		set_kmax();
 		return reset();
 	}
 
@@ -504,15 +539,27 @@ public:
 				   : wc == 4 ? (const void*)simplex_persistent_sharded<T, 4>
 				             : (const void*)simplex_persistent_sharded<T, 8>;
 		} else if (opt.pricing_rule == 1) {
-			fn = wc == 1 ? (const void*)simplex_persistent<T, 1, true>
-			   : wc == 2 ? (const void*)simplex_persistent<T, 2, true>
-			   : wc == 4 ? (const void*)simplex_persistent<T, 4, true>
-			             : (const void*)simplex_persistent<T, 8, true>;
+			if (d.kmax >= 0)
+				fn = wc == 1 ? (const void*)simplex_persistent<T, 1, true, true>
+				   : wc == 2 ? (const void*)simplex_persistent<T, 2, true, true>
+				   : wc == 4 ? (const void*)simplex_persistent<T, 4, true, true>
+				             : (const void*)simplex_persistent<T, 8, true, true>;
+			else
+				fn = wc == 1 ? (const void*)simplex_persistent<T, 1, true>
+				   : wc == 2 ? (const void*)simplex_persistent<T, 2, true>
+				   : wc == 4 ? (const void*)simplex_persistent<T, 4, true>
+				             : (const void*)simplex_persistent<T, 8, true>;
 		} else {
-			fn = wc == 1 ? (const void*)simplex_persistent<T, 1>
-			   : wc == 2 ? (const void*)simplex_persistent<T, 2>
-			   : wc == 4 ? (const void*)simplex_persistent<T, 4>
-			             : (const void*)simplex_persistent<T, 8>;
+			if (d.kmax >= 0)
+				fn = wc == 1 ? (const void*)simplex_persistent<T, 1, false, true>
+				   : wc == 2 ? (const void*)simplex_persistent<T, 2, false, true>
+				   : wc == 4 ? (const void*)simplex_persistent<T, 4, false, true>
+				             : (const void*)simplex_persistent<T, 8, false, true>;
+			else
+				fn = wc == 1 ? (const void*)simplex_persistent<T, 1>
+				   : wc == 2 ? (const void*)simplex_persistent<T, 2>
+				   : wc == 4 ? (const void*)simplex_persistent<T, 4>
+				             : (const void*)simplex_persistent<T, 8>;
 		}
 		CU(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(NT), args, DYN_SMEM_BYTES, stream));
 		launches++;
@@ -581,6 +628,25 @@ public:
 			res->kernel_launches = launches;
 		}
 		ms_run = 0;
+		return B200LP_OK;
+	}
+
+	int binv_info(int64_t* touched, int64_t* sparse_passes) override {
+		CU(cudaSetDevice(opt.device));
+		if (int rc = settle()) return rc;
+		Ctl t;
+		CU(cudaMemcpy(&t, d.ctl, sizeof(Ctl), cudaMemcpyDeviceToHost));
+		if (touched) *touched = d.kmask ? t.kcount : 0;
+		if (sparse_passes) *sparse_passes = t.kpasses;
+		return B200LP_OK;
+	}
+
+	int set_binv_sparse(int32_t k) override {
+		if (k < -1) return fail(B200LP_ERR_ARG, "binv_sparse must be -1 (off), 0 (auto) or a column count");
+		if (!d.kmask) return fail(B200LP_ERR_STATE, "binv_sparse: sharded engines stream all of B^-1");
+		if (int rc = settle()) return rc;
+		binv_sparse = k;
+		set_kmax();
 		return B200LP_OK;
 	}
 
@@ -755,11 +821,11 @@ public:
 
 	int download_vector(int32_t which, void* out) override {
 		const T* src = which == 0 ? d.alpha : which == 1 ? d.E_q : which == 2 ? d.row_q
-		             : which == 3 ? d.x_b : which == 4 ? d.y : which == 5 ? d.c_b : nullptr;
+		             : which == 3 ? d.x_b : which == 4 ? d.y : which == 5 ? d.c_b : which == 6 ? d.vbt : which == 7 ? d.gamma : nullptr;
 		if (!src || !out) return fail(B200LP_ERR_ARG, "download_vector: bad selector");
 		CU(cudaSetDevice(opt.device));
 		CU(cudaStreamSynchronize(stream));
-		CU(cudaMemcpy(out, src, d.m * sizeof(T), cudaMemcpyDeviceToHost));
+		CU(cudaMemcpy(out, src, (which == 7 ? d.n : d.m) * sizeof(T), cudaMemcpyDeviceToHost));
 		return B200LP_OK;
 	}
 
@@ -996,7 +1062,9 @@ private:
 		st->bar = 0;
 		st->price_ctr = st->upd_ctr = st->btran_ctr = 0;
 		st->xarr[0] = st->xarr[1] = 0;
-		cudaError_t e = cudaMemcpyAsync(d.ctl, st, sizeof(Ctl), cudaMemcpyHostToDevice, stream);
+		// everything up to the touched-column state, which only the device keeps (book1 replays of refactor and
+		// the phase entry points change it while hc is not pulled)
+		cudaError_t e = cudaMemcpyAsync(d.ctl, st, offsetof(Ctl, kcount), cudaMemcpyHostToDevice, stream);
 		if (e != cudaSuccess) return e;
 		// the staging buffer is reused: make sure the copy has been consumed
 		return cudaStreamSynchronize(stream);
@@ -1038,6 +1106,22 @@ private:
 		if (wc == 1) LAUNCH_UF(1); else if (wc == 2) LAUNCH_UF(2); else if (wc == 4) LAUNCH_UF(4); else LAUNCH_UF(8);
 #undef LAUNCH_UF
 		launches++;
+	}
+
+	// Touched-column passes of simplex_persistent (update_ftran_sparse): they run while ctl->kcount <= d.kmax.
+	// Auto: m >= KSPARSE_MIN_M and K* = m / 8.  Measured (DESIGN.md 3h, tools/sparse_binv_sweep.py): below m = 4096 the
+	// sparse passes cannot fill the grid and lose at every |K|; above it they win at every |K| reached, and the
+	// extrapolated crossovers lie at |K| >= m / 6.6.  An explicit K* skips the size gate.
+	void set_kmax() {
+		const bool auto_off = binv_sparse == 0 && d.m < KSPARSE_MIN_M;
+		d.kmax = (binv_sparse == -1 || auto_off || !d.kmask || d.nchunk > KACT_MAX || a_nonfinite || opt.fuse_ratio > 0) ? -1
+		       : binv_sparse > 0 ? (int)std::min<long long>(binv_sparse, d.m) : (int)(d.m / 8);
+	}
+
+	// a kernel changed B^-1 without book1_phase (simplex_tiny, simplex_resident): stream all of it until the next
+	// reset (any nonzero kdense; the control block's tail is device-owned, see push_ctl)
+	cudaError_t mark_dense() {
+		return cudaMemsetAsync(reinterpret_cast<unsigned char*>(d.ctl) + offsetof(Ctl, kdense), 0xff, sizeof(int), stream);
 	}
 
 	// the primal loop runs: algorithm = 0, or phase 2 of the composite method (algorithm = 1, cost_shift = 1)
@@ -1112,6 +1196,7 @@ private:
 	int run_resident(int64_t iters) {
 		hc.it_end = hc.iter + iters;
 		CU(push_ctl());
+		CU(mark_dense());
 		if (d.prof_cap > 0) CU(cudaMemsetAsync(d.prof, 0, (size_t)d.prof_cap * NSTAMP * sizeof(unsigned long long), stream));
 		prof_iter0 = hc.iter;
 		d.res_maxG = num_sms;
@@ -1129,6 +1214,7 @@ private:
 	int run_tiny(int64_t iters) {
 		hc.it_end = hc.iter + iters;
 		CU(push_ctl());
+		CU(mark_dense());
 		const size_t smem = TinyLayout<T>(d.m, d.n, d.ns).bytes(d.m);
 		CU(cudaFuncSetAttribute(simplex_tiny<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 		CU(cudaEventRecord(ev0, stream));
@@ -1195,6 +1281,9 @@ private:
 	int64_t launches = 0;
 	long long prof_iter0 = 0;
 	size_t l2_persist_bytes = 0;
+	int binv_sparse = 0;         // b200lp_set_binv_sparse
+	int* d_nonfinite = nullptr;  // k_flag_nonfinite's answer for the last upload
+	bool a_nonfinite = false;    // the stored columns hold an inf or NaN: fma(+0, a_j, acc) is not acc
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -1981,6 +2070,8 @@ int b200lp_phase_info(b200lp_engine* e, int32_t* phase, int64_t* shifted_columns
 	NEED(e);
 	return e->phase_info(phase, shifted_columns, phase1_pivots);
 }
+int b200lp_set_binv_sparse(b200lp_engine* e, int32_t k) { NEED(e); return e->set_binv_sparse(k); }
+int b200lp_binv_info(b200lp_engine* e, int64_t* touched, int64_t* sparse_passes) { NEED(e); return e->binv_info(touched, sparse_passes); }
 int b200lp_abort(b200lp_engine* e) { NEED(e); return e->abort(); }
 int b200lp_refactor(b200lp_engine* e, double rel_pivot_tol, int64_t* replayed) { NEED(e); return e->refactor(rel_pivot_tol, replayed); }
 

@@ -96,6 +96,13 @@ struct Ctl {
 	double min_e;             // last pricing minimum
 	double c_b_q;             // c_b[q] before the swap (v4:339)
 	double z;                 // c_b . x_b (v4:365)
+	// touched columns of B^-1 (Dev::kmask).  Device-owned: push_ctl stops in front of them, k_reset / k_identity clear
+	// them, the host only ever sets kdense (kernels that change B^-1 without book1_phase).
+	int kcount;               // columns whose mask bit is set
+	int kdense;               // the mask is not trusted (or a non-finite E_q was formed): stream all of B^-1 until a reset
+	int anf;                  // a sparse ratio phase met a non-finite alpha: the sparse BTRAN / passes are off until a reset
+	int pad1;
+	long long kpasses;        // update + FTRAN passes that streamed only the touched columns (b200lp_binv_info)
 };
 
 template <typename T>
@@ -150,6 +157,11 @@ struct Dev {
 	long long vpart_off;              // steepest edge, sharded: element offset (from alpha) of the R partial-v vectors in a mailbox
 	const T* dpart0;                  // row_q.b slice partials: dpart on one GPU, the mailbox's rqb when sharded
 	T* acol;                          // local copy of the entering column (sharded mode only)
+	// touched columns: bit j of kmask[j / 32] set = column j of B^-1 may differ from e_j (one word per FTRAN
+	// sub-block, nchunk * 8 words; nullptr when sharded).  kmax: simplex_persistent streams only the touched columns
+	// while ctl->kcount <= kmax; -1 = never (b200lp_set_binv_sparse(e, -1), fused ratio test, sharded, non-finite A, small m, ...)
+	unsigned int* kmask;
+	int kmax;
 };
 
 // head of a rank's mailbox; peers store into it over NVLink.  Every record carries its own flag
@@ -796,14 +808,35 @@ __device__ void price_phase_se(const Dev<T>& d, Smem& sh, const T* const (&vec)[
 
 // v = B^-T alpha: the column dots of B^-1 with alpha, in the pricing order (one extra read of B^-1 per pivot,
 // the price of exact steepest-edge weights).  Column groups come from ctl->btran_ctr.
+// sparse: only the touched columns get a dot (mask words w = part, part + nparts, ...).  An untouched column is e_j,
+// so every fma of its dot adds +0 to a +0-started chain and the dot is exactly 1 * alpha_j + 0 = alpha_j + 0 (alpha
+// finite: ctl->anf).  book1_phase may set the bit of this pivot's leaving row q concurrently; column q of B^-1 is
+// still e_q then, so either reading gives the same bits.
 template <typename T>
-__device__ void btran_phase(const Dev<T>& d, Smem& sh, const T* alpha_vec, int part, int nparts) {
+__device__ void btran_phase(const Dev<T>& d, Smem& sh, const T* alpha_vec, int part, int nparts, bool sparse = false) {
 	const int tid = threadIdx.x;
+	const T* const vec[3] = {alpha_vec, nullptr, nullptr};
+	int buf = 0;
+	if (sparse) {
+		for (long long w = part; w < (d.m + 31) / 32; w += nparts) {
+			__syncthreads();
+			if (tid == 0) sh.bc_c = __ldcg(d.kmask + w);      // one reading for the whole CTA (see above)
+			__syncthreads();
+			const unsigned kw = (unsigned)sh.bc_c;
+			const long long j = w * 32 + tid;
+			if (tid < 32 && j < d.m && !((kw >> tid) & 1u)) d.vbt[j] = alpha_vec[j] + T(0);
+			for (unsigned b = kw; b; b &= b - 1u, buf ^= 1) {
+				const long long col = w * 32 + __ffs(b) - 1;
+				column_dots<T, 1, 16, 1, true>(d.B + col * d.ldb, d.ldb, d.ldb, vec, sh, buf);
+				__syncthreads();
+				if (tid == 0) d.vbt[col] = warp_sums<T>(sh, buf, 0);
+			}
+		}
+		return;
+	}
 	const long long c1 = d.m;
 	const long long nq = c1 / PRICE_NC;
 	const long long nitems = nq + (c1 - nq * PRICE_NC);
-	const T* const vec[3] = {alpha_vec, nullptr, nullptr};
-	int buf = 0;
 	for (long long g = part; g < nitems; buf ^= 1) {
 		if (tid == 0) sh.tk = (long long)nparts + atomicAdd(&d.ctl->btran_ctr, 1u);
 		const bool quad = g < nq;
@@ -1104,13 +1137,213 @@ __device__ void update_ftran_phase(const Dev<T>& d, Smem& sh, unsigned char* dyn
 	}
 }
 
+// ---------------------------------------------------------------- touched columns only (simplex_persistent)
+//
+// Invariant: B^-1 starts as I and pivot k adds E_q (x) row_q with row_q = row q of the current B^-1.  Let K be the
+// leaving rows seen since the last reset (bits of Dev::kmask, set by book1_phase).  For a column j outside K,
+// row_q[j] = +0, so the update is fma(E_q[i], +0, B[i,j]) and leaves the column exactly e_j while E_q is finite.
+// So the update touches only K's columns, and in the FTRAN chains of the file header every other column adds
+// fma(+0, a_j, acc) = acc (a_p finite) except the unit term fma(1, a_i, acc) of row i's own column.  The sparse pass
+// below visits K's columns and those unit terms in column order, keeps the 8-way tree with explicit +0 sub-blocks
+// and writes the partials of the chunks that hold a K column ("active"); the ratio phase sums those, left to right,
+// with the unit term's chunk partial fma(1, a_i, +0) at chunk(i)'s place when that chunk is not active.  A chunk
+// partial left out is exactly +0, and x + (+0) = x.  Every result has the bits of the dense pass, except that a
+// zero may differ in sign when an fma chain underflows to -0 (only a chain that underflows can become -0).
+// The dense B^-1 in HBM stays the whole truth: untouched columns hold e_j there.
+
+constexpr int KACT_MAX = 1024;      // chunks the active list holds (m <= 262144); larger LPs stream all of B^-1
+constexpr long long KSPARSE_MIN_M = 4096;   // auto setting: smaller LPs stream all of B^-1 (measured, DESIGN.md 3h)
+
+// the active chunks of one pass, in shared memory of every CTA
+struct KAct {
+	int n;                          // active chunks
+	unsigned short c[KACT_MAX];     // their indices, ascending
+	unsigned int bit[KACT_MAX / 32];
+};
+
+// every CTA builds the list from the mask (nchunk * 8 words, read at L2 like row_q); warp 0 packs it in order
+template <typename T>
+__device__ void kact_build(const Dev<T>& d, KAct& ka) {
+	const int tid = threadIdx.x, lane = tid & 31;
+	const int nw = (d.nchunk + 31) / 32;
+	for (int w = tid; w < KACT_MAX / 32; w += NT) ka.bit[w] = 0u;
+	__syncthreads();
+	for (int c = tid; c < d.nchunk; c += NT) {
+		const uint4* p = reinterpret_cast<const uint4*>(d.kmask + (long long)c * (CHUNK / SUBW));
+		const uint4 a = __ldcg(p), b = __ldcg(p + 1);
+		if (a.x | a.y | a.z | a.w | b.x | b.y | b.z | b.w) atomicOr(&ka.bit[c >> 5], 1u << (c & 31));
+	}
+	__syncthreads();
+	if (tid < 32) {
+		const unsigned bw = lane < nw ? ka.bit[lane] : 0u;
+		int pos = __popc(bw);
+#pragma unroll
+		for (int off = 1; off < 32; off <<= 1) {              // inclusive scan of the popcounts
+			const int o = __shfl_up_sync(0xffffffffu, pos, off);
+			if (lane >= off) pos += o;
+		}
+		if (lane == 31) ka.n = pos;
+		pos -= __popc(bw);
+		for (unsigned b = bw; b; b &= b - 1u) ka.c[pos++] = (unsigned short)(lane * 32 + __ffs(b) - 1);
+	}
+	__syncthreads();
+}
+
+// The update + FTRAN pass of update_ftran_phase (WC = 1 tree, same bits) over the active chunks only.  Work items are
+// (row slab, active chunk), slab fastest, from ctl->upd_ctr; a thread owns SRS 16-byte row vectors NT vectors apart,
+// so every K column keeps SRS loads per thread in flight.  Rows whose own column lies in the chunk and is not in K
+// get their unit term at its place in the chain.  ka: kact_build of this pass.
+template <typename T, bool UPDATE>
+__device__ void update_ftran_sparse(const Dev<T>& d, Smem& sh, unsigned char* dyn, const KAct& ka, const T* acol, long long uk,
+		int part, int nparts) {
+	using M = Mem<T>;
+	using V = typename VecT<T>::V;
+	constexpr int VN = VecT<T>::N;
+	constexpr int SRS = 2;                                   // row steps per item
+	constexpr long long SLAB = (long long)SRS * NT * VN;
+	const int tid = threadIdx.x;
+	const long long ld = d.ldb, m = d.m;
+	const long long nslab = (ld + SLAB - 1) / SLAB;
+	const long long nitems = nslab * ka.n;
+	T* stage_rq = reinterpret_cast<T*>(dyn);
+	T* stage_a = reinterpret_cast<T*>(dyn + CHUNK * 8);
+	const bool unit = acol == nullptr;
+
+	for (long long ticket = part; ticket < nitems;) {
+		const long long sl = ticket % nslab, ck = ka.c[ticket / nslab];
+		const long long j0 = ck * CHUNK, r0 = sl * SLAB;
+		__syncthreads();
+		if (tid == 0) sh.tk = (long long)nparts + atomicAdd(&d.ctl->upd_ctr, 1u);
+		{
+			const long long j = j0 + tid;     // NT == CHUNK
+			T r = T(0), a = T(0);
+			if (j < m) {
+				if (UPDATE) r = __ldcg(d.row_q + j);
+				a = unit ? (j == uk ? T(1) : T(0)) : acol[j];
+			}
+			stage_rq[tid] = r;
+			stage_a[tid] = a;
+		}
+		__syncthreads();
+		ticket = sh.tk;
+
+		long long row[SRS];
+		V Ev[SRS];
+#pragma unroll
+		for (int u = 0; u < SRS; ++u) {
+			row[u] = r0 + (long long)u * NT * VN + (long long)tid * VN;
+			if (UPDATE && row[u] < ld) Ev[u] = *reinterpret_cast<const V*>(d.E_q + d.row0 + row[u]);
+		}
+		const bool diag = j0 < r0 + SLAB && r0 < j0 + CHUNK;   // some row of the slab has its own column in this chunk
+		T stk[4][SRS][VN];
+#pragma unroll
+		for (int s = 0; s < CHUNK / SUBW; ++s) {
+			const long long jb = j0 + s * SUBW;
+			T acc[SRS][VN];
+#pragma unroll
+			for (int u = 0; u < SRS; ++u)
+#pragma unroll
+				for (int v = 0; v < VN; ++v) acc[u][v] = T(0);
+			const unsigned kw = jb < m ? __ldcg(d.kmask + (jb >> 5)) : 0u;
+			unsigned uw = 0u;
+			if (diag) {
+#pragma unroll
+				for (int u = 0; u < SRS; ++u)
+#pragma unroll
+					for (int v = 0; v < VN; ++v) {
+						const long long i = row[u] + v;
+						if (i >= jb && i < jb + SUBW && i < m) uw |= 1u << (int)(i - jb);
+					}
+				uw = __reduce_or_sync(0xffffffffu, uw) & ~kw;
+			}
+			for (unsigned w = kw | uw; w; w &= w - 1u) {         // warp-uniform, columns in order
+				const int b = __ffs(w) - 1;
+				const T a = stage_a[s * SUBW + b];
+				if ((kw >> b) & 1u) {
+					const T r = stage_rq[s * SUBW + b];
+					T* bp = d.B + (jb + b) * ld;
+					V x[SRS];
+#pragma unroll
+					for (int u = 0; u < SRS; ++u)
+						if (row[u] < ld) x[u] = M::ld_stream(bp + row[u]);
+#pragma unroll
+					for (int u = 0; u < SRS; ++u) {
+						if (row[u] >= ld) continue;
+#pragma unroll
+						for (int v = 0; v < VN; ++v) {
+							T xv = M::get(x[u], v);
+							if (UPDATE) { xv = fma_t(M::get(Ev[u], v), r, xv); M::set(x[u], v, xv); }
+							acc[u][v] = fma_t(xv, a, acc[u][v]);
+						}
+						if (UPDATE) M::st_stream(bp + row[u], x[u]);
+					}
+				} else {                                         // B[i, i] = 1 for the row(s) whose column this is
+#pragma unroll
+					for (int u = 0; u < SRS; ++u)
+#pragma unroll
+						for (int v = 0; v < VN; ++v)
+							if (row[u] + v == jb + b) acc[u][v] = fma_t(T(1), a, acc[u][v]);
+				}
+			}
+			// the pairwise tree of update_ftran_phase (binary-counter stack)
+			int lvl = 0;
+#pragma unroll
+			for (; lvl < 3; ++lvl) {
+				if (!((s >> lvl) & 1)) break;
+#pragma unroll
+				for (int u = 0; u < SRS; ++u)
+#pragma unroll
+					for (int v = 0; v < VN; ++v) acc[u][v] = stk[lvl][u][v] + acc[u][v];
+			}
+#pragma unroll
+			for (int u = 0; u < SRS; ++u)
+#pragma unroll
+				for (int v = 0; v < VN; ++v) stk[lvl][u][v] = acc[u][v];
+		}
+#pragma unroll
+		for (int u = 0; u < SRS; ++u) {
+			if (row[u] >= ld) continue;
+			V o;
+#pragma unroll
+			for (int v = 0; v < VN; ++v) M::set(o, v, stk[3][u][v]);
+			*reinterpret_cast<V*>(d.alpha_part + ck * ld + row[u]) = o;
+		}
+	}
+}
+
+// alpha_i from the active chunks' partials, left to right, with the unit term's partial fma(1, a_i, +0) at chunk(i)'s
+// place when chunk(i) is not active (see above); the loads of 16 chunks are issued together like sum_chunk_partials
+template <typename T>
+__device__ __forceinline__ T sum_active_partials(const Dev<T>& d, const KAct& ka, long long i, const T* acol, long long uk) {
+	const int ci = (int)(i / CHUNK);
+	bool ins = !((ka.bit[ci >> 5] >> (ci & 31)) & 1u);
+	const T ut = ins ? fma_t(T(1), acol ? acol[i] : (i == uk ? T(1) : T(0)), T(0)) : T(0);
+	T a = T(0);
+	for (int k0 = 0; k0 < ka.n; k0 += 16) {
+		T v[16];
+#pragma unroll
+		for (int u = 0; u < 16; ++u) v[u] = k0 + u < ka.n ? __ldcg(d.alpha_part + (long long)ka.c[k0 + u] * d.ldb + i) : T(0);
+#pragma unroll
+		for (int u = 0; u < 16; ++u) {
+			if (k0 + u >= ka.n) break;
+			if (ins && ka.c[k0 + u] > ci) { a = a + ut; ins = false; }
+			a = a + v[u];
+		}
+	}
+	if (ins) a = a + ut;
+	return a;
+}
+
 // ---------------------------------------------------------------- phase: ratio test
 
 // alpha_i = sum of the chunk partials (left to right); theta_i = x_b_i/alpha_i
 // over alpha_i > 0 (strict, v4:203); masked argmin + eligible-row count.
 // Replaces cudaMemset + compute_theta + D2H + cub ArgMin (v4:311-325).
+// ka: the pass was update_ftran_sparse (entering column acol, or e_uk when acol is null); a non-finite alpha then
+// sets ctl->anf.
 template <typename T, bool FROM_PARTIALS>
-__device__ void ratio_phase(const Dev<T>& d, Smem& sh, int part, int nparts, T* stage = nullptr) {
+__device__ void ratio_phase(const Dev<T>& d, Smem& sh, int part, int nparts, T* stage = nullptr,
+		const KAct* ka = nullptr, const T* acol = nullptr, long long uk = 0) {
 	const int tid = threadIdx.x;
 	double best_v = CUDART_INF;
 	long long best_i = LLONG_MAX;
@@ -1125,7 +1358,16 @@ __device__ void ratio_phase(const Dev<T>& d, Smem& sh, int part, int nparts, T* 
 		}
 	};
 	const long long nblk = (d.m + 31) / 32;
-	if (FROM_PARTIALS && stage && nblk <= 2 * (long long)nparts) {
+	if (FROM_PARTIALS && ka) {
+		bool bad = false;
+		for (long long i = (long long)part * NT + tid; i < d.m; i += (long long)nparts * NT) {
+			const T a = sum_active_partials<T>(d, *ka, i, acol, uk);
+			d.alpha[i] = a;
+			bad |= !isfinite(a);
+			consider(i, a);
+		}
+		if (bad) d.ctl->anf = 1;
+	} else if (FROM_PARTIALS && stage && nblk <= 2 * (long long)nparts) {
 		// blocks of 32 rows, the CTA's warps load the chunk partials together (sum_partials_rows32); only while
 		// every CTA gets at most two blocks (measured at m = 32768 on one GPU, 3.5 blocks per CTA: 20.7 us against
 		// 12.8 us for one row per thread)
@@ -1204,10 +1446,15 @@ __device__ void book1_phase(const Dev<T>& d, Smem& sh, long long p, long long q,
 			const T eq = (i != q) ? (-al / alpha_q) : (T)(1.0 / (double)alpha_q - 1.0);
 			d.row_q[i] = rq;
 			d.E_q[i] = eq;
+			if (!isfinite(eq)) d.ctl->kdense = 1;       // fma(inf, +0, .) = NaN: untouched columns would change too
 			T cb = d.c_b[i];
 			if (i == q) {
 				d.ctl->c_b_q = (double)cb; cb = c_p;
 				if (SE) { d.ctl->alpha_q = (double)alpha_q; d.ctl->leaving = d.b_ixs[q]; }
+				if (d.kmask) {                           // column q joins the touched set (the only writer of the word)
+					const unsigned w = __ldcg(d.kmask + (q >> 5)), bit = 1u << (q & 31);
+					if (!(w & bit)) { d.kmask[q >> 5] = w | bit; d.ctl->kcount = __ldcg(&d.ctl->kcount) + 1; }
+				}
 			}
 			t1 = fma_t(rq, d.b[i], T(0));
 			t2 = fma_t(cb, eq, T(0));
@@ -1348,9 +1595,13 @@ __device__ double objective(const Dev<T>& d, Smem& sh) {
 // book2 stays a phase of its own with a fourth barrier.
 // SE: steepest-edge pricing (price_phase_se), one more read of B^-1 per pivot for v = B^-T alpha (btran_phase, in
 // the same barrier interval as book1).
-template <typename T, int WC, bool SE = false>
+// KS: the loop may take the touched-column passes (update_ftran_sparse, the sparse ratio phase and BTRAN); the host
+// launches this instantiation only when d.kmax >= 0.  KS = false compiles none of that code, so the dense loop keeps its
+// register allocation (the sparse passes raise the kernel's spills, which costs the pricing pass of small LPs).
+template <typename T, int WC, bool SE = false, bool KS = false>
 __global__ void __launch_bounds__(NT, MIN_CTAS) simplex_persistent(Dev<T> d) {
 	__shared__ Smem sh;
+	__shared__ KAct ka;                 // active chunks of the current sparse pass (update + FTRAN, ratio)
 	extern __shared__ __align__(128) unsigned char ringbuf[];
 	Ring rcons, rprod;
 	ring_init(sh, rcons, rprod, d.price_nc);
@@ -1415,6 +1666,10 @@ __global__ void __launch_bounds__(NT, MIN_CTAS) simplex_persistent(Dev<T> d) {
 		const T* acol = p < d.ns ? d.A + p * d.ld : nullptr;
 		double th;
 		long long elig;
+		// touched columns only (never with fuse_ratio: the host sets kmax = -1): the same bits (see
+		// update_ftran_sparse), decided from state every CTA reads after B1
+		const bool ksp = KS && d.kmax >= 0 && !__ldcg(&ctl->kdense) && !__ldcg(&ctl->anf) && __ldcg(&ctl->kcount) <= d.kmax;
+		bool kbt = false;                   // sparse BTRAN of this pivot (steepest edge): alpha is finite as well
 		if (d.fuse_ratio) {
 			if (pending) update_ftran_phase<T, WC, true, true, true>(d, sh, ringbuf, acol, p - d.ns, pivots & 1, me, G);
 			else         update_ftran_phase<T, WC, false, true, true>(d, sh, ringbuf, acol, p - d.ns, pivots & 1, me, G);
@@ -1425,14 +1680,21 @@ __global__ void __launch_bounds__(NT, MIN_CTAS) simplex_persistent(Dev<T> d) {
 			reduce_cands(d.rcand, d.ngrp, th, q, sh);
 			elig = reduce_counts(d.rcnt, d.ngrp, sh);
 		} else {
-			if (pending) update_ftran_phase<T, WC, true, true, false>(d, sh, ringbuf, acol, p - d.ns, pivots & 1, me, G);
-			else         update_ftran_phase<T, WC, false, true, false>(d, sh, ringbuf, acol, p - d.ns, pivots & 1, me, G);
+			if (ksp) {
+				if (me == 0 && threadIdx.x == 0) ctl->kpasses += 1;
+				kact_build<T>(d, ka);
+				if (pending) update_ftran_sparse<T, true>(d, sh, ringbuf, ka, acol, p - d.ns, me, G);
+				else         update_ftran_sparse<T, false>(d, sh, ringbuf, ka, acol, p - d.ns, me, G);
+			} else if (pending) update_ftran_phase<T, WC, true, true, false>(d, sh, ringbuf, acol, p - d.ns, pivots & 1, me, G);
+			else                update_ftran_phase<T, WC, false, true, false>(d, sh, ringbuf, acol, p - d.ns, pivots & 1, me, G);
 			stamp(d, it - it0, 3);
 			grid_barrier(ctl, epoch, G);
 			if (me == 0 && threadIdx.x == 0) ctl->upd_ctr = 0;
-			ratio_phase<T, true>(d, sh, me, G, reinterpret_cast<T*>(ringbuf));
+			if (ksp) ratio_phase<T, true>(d, sh, me, G, nullptr, &ka, acol, p - d.ns);
+			else     ratio_phase<T, true>(d, sh, me, G, reinterpret_cast<T*>(ringbuf));
 			grid_barrier(ctl, epoch, G);
 			stamp(d, it - it0, 4);
+			kbt = SE && ksp && !__ldcg(&ctl->anf);
 			reduce_cands(d.cand, G, th, q, sh);
 			elig = reduce_counts(d.cnt, G, sh);
 			if (d.ratio_mode == 2 && elig > 0) {        // Harris: th is theta_max, now pick the largest pivot inside it
@@ -1448,7 +1710,7 @@ __global__ void __launch_bounds__(NT, MIN_CTAS) simplex_persistent(Dev<T> d) {
 
 		// ---- pivot (v4:331-356)
 		book1_phase<T, SE>(d, sh, p, q, me, G);
-		if (SE) { btran_phase<T>(d, sh, d.alpha, me, G); pendg = true; }
+		if (SE) { btran_phase<T>(d, sh, d.alpha, me, G, kbt); pendg = true; }
 		stamp(d, it - it0, 6);
 		grid_barrier(ctl, epoch, G);
 		stamp(d, it - it0, 7);
@@ -3085,12 +3347,23 @@ __global__ void k_copy(T* dst, const T* src, long long n) {
 	for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) dst[i] = src[i];
 }
 
+// B^-1 = I: no column touched (Dev::kmask, Ctl::kcount / kdense / anf)
+template <typename T>
+__device__ __forceinline__ void k_clear_touched(const Dev<T>& d) {
+	if (!d.kmask) return;
+	for (long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x; w < (long long)d.nchunk * (CHUNK / SUBW);
+			w += (long long)gridDim.x * blockDim.x)
+		d.kmask[w] = 0u;
+	if (blockIdx.x == 0 && threadIdx.x == 0) { d.ctl->kcount = 0; d.ctl->kdense = 0; d.ctl->anf = 0; d.ctl->kpasses = 0; }
+}
+
 // B^-1 = I on the local row block (start of a refactorisation; the O(m) vectors stay)
 template <typename T>
 __global__ void k_identity(Dev<T> d) {
 	const long long tot = d.ldb * d.m;
 	for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < tot; e += (long long)gridDim.x * blockDim.x)
 		d.B[e] = (d.row0 + e % d.ldb == e / d.ldb) ? T(1) : T(0);
+	k_clear_touched(d);
 }
 
 template <typename T>
@@ -3151,6 +3424,15 @@ __global__ void __launch_bounds__(NT) k_gamma_init(Dev<T> d) {
 	for (long long k = d.k0 + (long long)blockIdx.x * NT + tid; k < d.k1; k += (long long)gridDim.x * NT) d.gamma[d.ns + k] = T(2);
 }
 
+// *flag = 1 when a[0..n) holds an inf or NaN (uploaded columns; the touched-column passes need a finite a_p)
+template <typename T>
+__global__ void k_flag_nonfinite(const T* a, long long n, int* flag) {
+	bool bad = false;
+	for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+		bad |= !isfinite(a[i]);
+	if (__syncthreads_or(bad) && threadIdx.x == 0) *flag = 1;
+}
+
 // slack-basis initial state (v4:272-277): B^-1 = I, c_b = c[n-m..n), x_b = b,
 // b_ixs[j] = n-m+j, y = c_b; padding rows zero.
 template <typename T>
@@ -3172,6 +3454,7 @@ __global__ void k_reset(Dev<T> d) {
 		d.row_q[i] = T(0);
 		if (in) d.b_ixs[i] = (int)(d.n - d.m + i);
 	}
+	k_clear_touched(d);
 }
 
 // nonbasic mask of the slack basis (dual simplex): the first n - m columns are nonbasic, the last m basic

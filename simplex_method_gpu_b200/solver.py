@@ -194,8 +194,10 @@ class Engine:
     """Handle API: device state survives between calls (benchmark windows, phase tests)."""
 
     def __init__(self, m: int, n: int, dtype=np.float64, eps: float = EPS, max_iter: int = MAX_ITER,
-                 device: int = 0, devices=None, **opts):
-        """``devices``: list of CUDA ordinals -> one handle over several GPUs of this process (b200lp_create_multi)."""
+                 device: int = 0, devices=None, binv_sparse: int = 0, **opts):
+        """``devices``: list of CUDA ordinals -> one handle over several GPUs of this process (b200lp_create_multi).
+        ``binv_sparse``: touched-column passes over B^-1 (b200lp_set_binv_sparse): 0 auto, -1 off, > 0 the largest
+        touched-column count they run at."""
         self.m, self.n, self.dtype = int(m), int(n), np.dtype(dtype)
         self._L = capi.lib()
         self._o = capi.default_options(eps=eps, max_iter=int(max_iter), device=device, **opts)
@@ -206,6 +208,18 @@ class Engine:
                                                    C.byref(self._o), C.byref(self._h)))
         else:
             capi.check(self._L.b200lp_create(_dtype_code(self.dtype), self.m, self.n, C.byref(self._o), C.byref(self._h)))
+        if binv_sparse != 0:
+            self.set_binv_sparse(binv_sparse)
+
+    def set_binv_sparse(self, k: int):
+        """Touched-column passes over B^-1 from the next run on: 0 auto, -1 off, > 0 while at most k columns are touched."""
+        capi.check(self._L.b200lp_set_binv_sparse(self._h, int(k)))
+
+    def binv_info(self) -> dict:
+        """Touched columns of B^-1 since the last reset / refactor and the update passes that streamed only them."""
+        k, n = C.c_int64(0), C.c_int64(0)
+        capi.check(self._L.b200lp_binv_info(self._h, C.byref(k), C.byref(n)))
+        return {"touched": k.value, "sparse_passes": n.value}
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
@@ -300,8 +314,8 @@ class Engine:
         return buf[:k.value].copy()
 
     def vector(self, name: str) -> np.ndarray:
-        which = {"alpha": 0, "E_q": 1, "row_q": 2, "x_b": 3, "y": 4, "c_b": 5}[name]
-        out = np.zeros(self.m, self.dtype)
+        which = {"alpha": 0, "E_q": 1, "row_q": 2, "x_b": 3, "y": 4, "c_b": 5, "vbt": 6, "gamma": 7}[name]
+        out = np.zeros(self.n if name == "gamma" else self.m, self.dtype)
         capi.check(self._L.b200lp_download_vector(self._h, which, _vp(out)))
         return out
 

@@ -34,6 +34,7 @@ ap.add_argument("--tail", type=int, default=0, help="price_tail: 0 auto, -1 none
 ap.add_argument("--fuse", type=int, default=0, help="fuse_book2: 0 auto, -1 off")
 ap.add_argument("--fuse-ratio", type=int, default=0, help="fuse_ratio: 0 auto, -1 off")
 ap.add_argument("--rule", type=int, default=0, help="pricing_rule: 0 Dantzig, 1 steepest edge")
+ap.add_argument("--binv-sparse", type=int, default=0, help="binv_sparse: 0 auto, -1 off (stream all of B^-1), else K*")
 ap.add_argument("--resident", type=int, default=0, help="1: label the stamps of the shared-memory-resident kernel (mid-size LPs, auto configuration)")
 ap.add_argument("--out", default="")
 a = ap.parse_args()
@@ -59,7 +60,8 @@ if world > 1:
     names = names["sharded"]
 else:
     e = lp.Engine(a.m, a.n, np.float64, eps=1e-9, max_iter=1 << 30, profile=a.pivots, grid_ctas=a.grid, tile_shape=a.shape, price_cols=a.price_cols, l2_persist_mb=a.l2, price_mode=a.price_mode,
-                      ratio_group_rows=a.group_rows, price_tail=a.tail, fuse_book2=a.fuse, fuse_ratio=a.fuse_ratio, pricing_rule=a.rule)
+                      ratio_group_rows=a.group_rows, price_tail=a.tail, fuse_book2=a.fuse, fuse_ratio=a.fuse_ratio, pricing_rule=a.rule,
+                      binv_sparse=a.binv_sparse)
     e.generate_dense(1)
     names = names["resident"] if a.resident else names["single"]
 
